@@ -44,6 +44,28 @@ def sample_step(utils_mod, data, batch, seed):
                                                        NEG, "uniform")
 
 
+DUMP_MAX_ELEMS = 15 << 20       # float32 elements of one dump: 60 MiB in all, below 64 MB with the .npy headers
+
+
+def dump_step_outputs(out_dir, loss, model):
+    """--dump-outputs: what the timed train step hands its caller after its last step - the loss, and every
+    parameter as Adam left it with the gradient it was updated from - as <out_dir>/<name>.npy in float32 (loss:
+    float64).  When these arrays hold more than DUMP_MAX_ELEMS elements together, each is written as the same seeded
+    sample of the same share of its flattened elements in every run, so that two builds can be compared output for
+    output."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = [("param." + name, p) for name, p in model.named_parameters()]
+    arrays += [("grad." + name, p.grad) for name, p in model.named_parameters() if p.grad is not None]
+    share = min(1.0, DUMP_MAX_ELEMS / sum(t.numel() for _, t in arrays))
+    np.save(os.path.join(out_dir, "loss.npy"), np.asarray([float(loss)], dtype=np.float64))
+    for name, t in arrays:
+        a = t.detach().float().cpu().numpy().reshape(-1)
+        keep = int(a.size * share)
+        if keep < a.size:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -977,7 +999,15 @@ def run_gpu(args):
     launches = L.launches
     prof, L.profile = L.profile, None
     restore(snap)
-    ms_eager = max_over_ranks(timed(lambda: step(resident), args.steps))
+    last_eager_loss = []
+
+    def eager_step():
+        # detached: an autograd graph that outlives its step would make the capture below fail
+        last_eager_loss[:] = [step(resident).detach()]
+
+    ms_eager = max_over_ranks(timed(eager_step, args.steps))
+    if args.dump_outputs and args.eager and rank == 0:
+        dump_step_outputs(args.dump_outputs, last_eager_loss[0], model)
     sync_all()
     restore(snap)
     captured = None
@@ -991,6 +1021,8 @@ def run_gpu(args):
         restore(snap)
         launches = captured.launches_per_step * args.steps
         ms_dev = max_over_ranks(timed(lambda: captured.step(), args.steps))
+        if args.dump_outputs and rank == 0:
+            dump_step_outputs(args.dump_outputs, captured.loss, model)
 
         def step(t):                                            # e2e: new inputs copied into place, then the replay
             return captured.step(node_id=t["node_id"], src=t["src"], dst=t["dst"], etype=t["etype"], norm=t["norm"],
@@ -1049,9 +1081,8 @@ def run_gpu(args):
             " ".join(f"{v:.4f}" for v in sampler_losses))
         cap2.close()
         sync_all()
-    n_host = 3
-    ms_host_sampler = max_over_ranks(timed_with_host_sampler(n_host, threaded=False)) / n_host
-    ms_host_threaded = max_over_ranks(timed_with_host_sampler(n_host, threaded=True)) / n_host
+    ms_host_sampler = max_over_ranks(timed_with_host_sampler(args.steps, threaded=False)) / args.steps
+    ms_host_threaded = max_over_ranks(timed_with_host_sampler(args.steps, threaded=True)) / args.steps
     sync_all()
 
     # ---- L2 throughput of this GPU for whole-row gathers / reductions (roofline denominator) --------
@@ -1148,7 +1179,7 @@ def run_gpu(args):
         # the peer-memory gather measured 2.4x slower at N = 8 (profiles/r02f): only on request (--peer)
         legs = (("single", True),) if world == 1 else ((("allgather", True), ("peer", False)) if args.peer else (("allgather", True),))
         for name, ag in legs:
-            partitioned["modes"][name] = partitioned_leg(args, dev, world, rank, log, allgather=ag, steps=3, warmup=3,
+            partitioned["modes"][name] = partitioned_leg(args, dev, world, rank, log, allgather=ag, steps=args.steps, warmup=3,
                                                          scale=args.scale)
             log(f"  [wikikg2-part x{world}, {name}] {partitioned['modes'][name]['ms_per_step']:.1f} ms/step")
         best = min(partitioned["modes"].values(), key=lambda m: m["ms_per_step"])
@@ -1332,7 +1363,9 @@ def run_gpu(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of every train-step and evaluation loop on the GPU; the CPU baseline (2 steps) "
+                         "and the GEMM, L2 and streaming probes keep their fixed repetition counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="fb15k237-full",
@@ -1361,7 +1394,13 @@ def main():
                     help="run only the wikikg2-shaped message-passing leg (profiling aid; prints its JSON object)")
     ap.add_argument("--no-streaming", action="store_true",
                     help="skip the wikikg2-shaped message-passing leg (HBM-streaming regime, N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss, parameters and gradients to DIR/<name>.npy "
+                         "(link-prediction workloads of this repo's CUDA path)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.streaming_only or args.workload in ("wikikg2-part", "am-entity")):
+        ap.error("--dump-outputs writes the outputs of the link-prediction train step: use it with --impl b200 and a "
+                 "fb15k237-* / wn18-* workload")
     global BASES
     BASES = args.bases if args.bases else (25 if args.workload.startswith("wn18") else 100)
     if args.streaming_only:

@@ -15,7 +15,11 @@ def pytest_configure(config):
 
 
 def load_golden(name):
-    return dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+    gv = dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+    if "inputs_sha256" in gv:
+        from helpers import redraw_inputs
+        gv.update(redraw_inputs(gv))
+    return gv
 
 
 @pytest.fixture(scope="session")

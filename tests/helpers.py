@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests (oracle side only - never imported by the package)."""
+import hashlib
 import os
 import sys
 
@@ -29,6 +30,53 @@ def rel_err(a, b):
 def assert_close(a, b, rtol=RTOL, what=""):
     e = rel_err(a, b)
     assert e <= rtol, f"{what}: relative error {e:.3e} > {rtol:.1e}"
+
+
+def at_golden_rows(gv, key, t):
+    """The rows of ``t`` that golden case ``gv`` keeps of output ``key``: all of them, unless the case stores a
+    seeded sample of the rows (``rows/<key>``) to stay small."""
+    rows = gv.get("rows/" + key)
+    return t if rows is None else t[torch.as_tensor(rows)]
+
+
+# A golden case too large to store whole (kgvae_small_noflow) leaves out the random inputs of its reference run and
+# keeps the SHA-256 of them instead; they are drawn again here from the case's seed, in the order the run drew them:
+# parameter initialisation (embedding, the two bdd layers, MoG prior, relation matrix), bias noise, eps, dropout
+# masks, then the evaluation pass's eps.
+REDRAWN = ["param/encoder.input_layer.embedding.weight", "param/encoder.rconv_layer_1.weight",
+           "param/encoder.rconv_layer_1.loop_weight", "param/encoder.rconv_layer_2.weight",
+           "param/encoder.rconv_layer_2.loop_weight", "param/encoder.z_pre", "param/w_relation",
+           "param/encoder.rconv_layer_1.h_bias", "param/encoder.rconv_layer_2.h_bias",
+           "eps", "mask1", "mask2", "eval_eps"]
+
+
+def inputs_sha256(arrays):
+    h = hashlib.sha256()
+    for key in REDRAWN:
+        h.update(np.ascontiguousarray(arrays[key]).tobytes())
+    return h.hexdigest()
+
+
+def redraw_inputs(gv):
+    """REDRAWN of a case without IAF flows, checked against the digest the case recorded."""
+    n_ent, n_rel, h, bases, k, n_flows, _ = (int(x) for x in gv["cfg"])
+    assert n_flows == 0
+    keep = 1.0 - float(gv["cfg_f"][2])
+    n, si = len(gv["node_id"]), h // bases
+    g = torch.Generator().manual_seed(int(gv["seed"]))
+    xavier = lambda *shape: torch.nn.init.xavier_uniform_(torch.empty(*shape), torch.nn.init.calculate_gain("relu"),
+                                                          generator=g)
+    drawn = [torch.empty(n_ent, h).normal_(generator=g),
+             xavier(2 * n_rel, bases * si * si), xavier(h, h), xavier(2 * n_rel, bases * si * 2 * si), xavier(h, 2 * h),
+             torch.randn(1, 2 * k, h, generator=g) / np.sqrt(k * h)]
+    drawn += [xavier(n_rel, h), torch.zeros(h).normal_(0, 0.1, generator=g), torch.zeros(2 * h).normal_(0, 0.1, generator=g),
+              torch.randn(n, h, generator=g)]
+    drawn += [(torch.rand(n, w, generator=g) < keep).float() / keep for w in (h, 2 * h)]
+    drawn.append(torch.randn(n_ent, h, generator=g))
+    out = {key: t.numpy() for key, t in zip(REDRAWN, drawn)}
+    assert inputs_sha256(out) == str(gv["inputs_sha256"]), \
+        "torch's random stream no longer reproduces the inputs this golden case was recorded with"
+    return out
 
 
 def golden_params(gv, requires_grad=False):

@@ -200,23 +200,26 @@ def made_masks(input_size, hidden_size, n_hidden):
     return masks
 
 
-def made_net(x, weights, biases, masks):
+def made_net(x, weights, biases, masks, relu_patterns=None):
+    """``relu_patterns`` (optional): one bool mask per hidden layer ([N, hidden] or a [1, hidden] row that
+    broadcasts) naming the units that count as active, in place of ``pre-activation > 0`` - see kgvae_encode."""
     n = len(weights)
     for i in range(n):
         x = F.linear(x, masks[i] * weights[i], biases[i])     # flow_network.py:15
         if i + 1 < n:
-            x = torch.relu(x)
+            x = torch.relu(x) if relu_patterns is None else torch.where(relu_patterns[i], x, torch.zeros_like(x))
     return x
 
 
-def made_forward(z, weights, biases, masks, degrees):
+def made_forward(z, weights, biases, masks, degrees, relu_patterns=None):
     """``len(degrees)`` full passes; pass p overwrites columns ``degrees[p]`` with
     ``z * exp(alpha + mu)``; log-det is the row-sum of the last pass's alpha
-    (flow_network.py:91-96)."""
+    (flow_network.py:91-96).  ``relu_patterns`` (optional): per pass, the list made_net takes."""
     x = torch.zeros_like(z)
     alpha = None
-    for idx in degrees:
-        mu, alpha = torch.chunk(made_net(x, weights, biases, masks), 2, dim=1)
+    for p, idx in enumerate(degrees):
+        pattern = None if relu_patterns is None else relu_patterns[p]
+        mu, alpha = torch.chunk(made_net(x, weights, biases, masks, pattern), 2, dim=1)
         x = x.clone()
         x[:, idx] = z[:, idx] * torch.exp(alpha[:, idx] + mu[:, idx])
     return x, alpha.sum(-1)
@@ -237,15 +240,17 @@ def flow_params(params, n_flows):
     return out
 
 
-def iaf_forward(z, params, n_flows):
+def iaf_forward(z, params, n_flows, made_relu_patterns=None):
     """MADE, reverse columns, MADE, ...; scalar ``flow_log_prob`` is the mean over
-    nodes of the summed log-dets (reference kgvae/model.py:115-123)."""
+    nodes of the summed log-dets (reference kgvae/model.py:115-123).
+    ``made_relu_patterns`` (optional): per MADE, the per-pass lists made_forward takes."""
     h = z.shape[1]
     masks = made_masks(h, h, n_flows)
     degs = made_degrees(h, h, n_flows)
     log_det_sum = torch.zeros(z.shape[0], dtype=z.dtype)
-    for ws, bs in flow_params(params, n_flows):
-        z, log_det = made_forward(z, ws, bs, masks, degs)
+    for f, (ws, bs) in enumerate(flow_params(params, n_flows)):
+        pattern = None if made_relu_patterns is None else made_relu_patterns[f]
+        z, log_det = made_forward(z, ws, bs, masks, degs, pattern)
         log_det_sum = log_det_sum + log_det
         z = z.flip(1)                                          # flow_network.py:28-30
     return z, log_det_sum, log_det_sum.view(-1, 1).mean()
@@ -254,12 +259,15 @@ def iaf_forward(z, params, n_flows):
 # ---------------------------------------------------------------------------
 # a2 + a3 + a5 + a6  encoder        reference kgvae/model.py:107-124
 # ---------------------------------------------------------------------------
-def kgvae_encode(params, graph, node_id, eps, num_bases, n_flows=0, drop_masks=(None, None), relu_pattern=None):
+def kgvae_encode(params, graph, node_id, eps, num_bases, n_flows=0, drop_masks=(None, None), relu_pattern=None,
+                 made_relu_patterns=None):
     """``relu_pattern`` (bool [N, h], optional): which units of layer 1 count as active.  ReLU has no derivative
     at 0, and a pre-activation within rounding error of 0 can land on either side depending on the summation
     order; a gradient comparison at millions of units (the benchmark-size parity test) hands the other
     implementation's pattern in here so that both sides differentiate the same piecewise-linear function.
-    The forward value changes by at most the magnitude of those pre-activations (~1e-6)."""
+    The forward value changes by at most the magnitude of those pre-activations (~1e-6).
+    ``made_relu_patterns`` (optional): the same for the hidden layers of the IAF flow - per MADE, per pass, per
+    hidden layer a bool mask ([N, h], or [1, h] for a pass whose rows are all equal, such as the first)."""
     p = params
     h0 = p["encoder.input_layer.embedding.weight"][torch.as_tensor(node_id).view(-1)]
     act1 = torch.relu if relu_pattern is None else (lambda t: t * relu_pattern.to(t.dtype))
@@ -275,7 +283,7 @@ def kgvae_encode(params, graph, node_id, eps, num_bases, n_flows=0, drop_masks=(
     z0 = sample_gaussian(z_mean, z_sigma, eps)
     out = {"h0": h0, "h1": h1, "h2": h2, "z_mean": z_mean, "z_sigma": z_sigma, "z0": z0}
     if n_flows > 0:
-        z, lds, flp = iaf_forward(z0, params, n_flows)
+        z, lds, flp = iaf_forward(z0, params, n_flows, made_relu_patterns)
         out.update(z=z, log_det_sum=lds, flow_log_prob=flp)
     else:
         out.update(z=z0, log_det_sum=None, flow_log_prob=None)

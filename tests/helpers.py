@@ -99,6 +99,36 @@ def golden_graph(gv, prefix="g_", etype_key="edge_type", norm_key="node_norm", n
             "edge_norm": norm[dst].reshape(-1, 1)}
 
 
+def made_relu_patterns(z, weights, biases, masks, degrees, against=None):
+    """The plain oracle MADE forward (O.made_forward without a pattern), replayed pass by pass to expose the hidden
+    layers.  Returns (x, patterns, flips): ``patterns[p][l]`` is ``pre-activation > 0`` of hidden layer l in pass p,
+    the nesting ``O.made_forward(relu_patterns=...)`` takes.  ``against``: another implementation's patterns, same
+    nesting (a pass may give one [1, h] row for all rows, as the first pass does on the GPU); then ``flips`` is
+    (number of units whose sign differs, largest |pre-activation| among them relative to its layer's largest)."""
+    import torch.nn.functional as F
+    x = torch.zeros_like(z)
+    patterns, n_flip, worst = [], 0, 0.0
+    for p, idx in enumerate(degrees):
+        h, layer = x, []
+        for i in range(len(weights)):
+            h = F.linear(h, masks[i] * weights[i], biases[i])
+            if i + 1 < len(weights):
+                layer.append(h > 0)
+                if against is not None:
+                    other = against[p][i].to(h.device)
+                    pre = h[:other.shape[0]]
+                    diff = other != (pre > 0)
+                    if bool(diff.any()):
+                        n_flip += int(diff.sum())
+                        worst = max(worst, float(pre.abs()[diff].max() / pre.abs().max()))
+                h = torch.relu(h)
+        mu, alpha = torch.chunk(h, 2, dim=1)
+        x = x.clone()
+        x[:, idx] = z[:, idx] * torch.exp(alpha[:, idx] + mu[:, idx])
+        patterns.append(layer)
+    return x, patterns, (n_flip, worst)
+
+
 def oracle_train_step(gv, requires_grad=True):
     """Run the oracle port on a golden case's inputs; returns (params, enc, loss dict)."""
     n_ent, n_rel, h, bases, k, n_flows, neg = (int(x) for x in gv["cfg"])

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import O, assert_close, at_golden_rows, golden_graph, golden_params, oracle_train_step
+from helpers import O, assert_close, at_golden_rows, golden_graph, golden_params, made_relu_patterns, oracle_train_step
 
 CASES = ["kgvae_tiny_noflow", "kgvae_tiny_flow3", "kgvae_small_noflow"]
 
@@ -140,6 +140,74 @@ def test_made_block(golden):
     zi, ldi = O.made_inverse(x.detach(), [w.detach() for w in ws], [b.detach() for b in bs], masks)
     assert_close(zi, gv["inv_z"], 1e-5, "inverse z")
     assert_close(ldi, gv["inv_log_det"], 1e-5, "inverse log_det")
+
+
+def test_made_relu_patterns_are_the_plain_function(golden):
+    """``relu_patterns`` / ``made_relu_patterns``: handed the oracle's own ReLU pattern, the oracle computes the plain
+    function bit for bit (forward and every gradient, one MADE and a two-MADE flow); with one unit flipped, only the
+    row that unit belongs to changes."""
+    gv = golden("made_block")
+    D, nh, N = (int(x) for x in gv["cfg"])
+    masks, degs = O.made_masks(D, D, nh), O.made_degrees(D, D, nh)
+    W = [torch.from_numpy(gv[f"param/net.{2 * l}.weight"]).double() for l in range(nh + 2)]
+    B = [torch.from_numpy(gv[f"param/net.{2 * l}.bias"]).double() for l in range(nh + 2)]
+    Z = torch.from_numpy(gv["z"]).double()
+    gen = torch.Generator().manual_seed(3)
+    gx, gl = torch.randn(N, D, generator=gen, dtype=torch.float64), torch.randn(N, generator=gen, dtype=torch.float64)
+
+    def run(patterns):
+        ws, bs = [t.clone().requires_grad_(True) for t in W], [t.clone().requires_grad_(True) for t in B]
+        z = Z.clone().requires_grad_(True)
+        x, log_det = O.made_forward(z, ws, bs, masks, degs, patterns)
+        ((x * gx).sum() + (log_det * gl).sum()).backward()
+        return [x.detach(), log_det.detach(), z.grad] + [t.grad for t in ws + bs]
+
+    plain = run(None)
+    x_replay, pats, _ = made_relu_patterns(Z, W, B, masks, degs)
+    assert torch.equal(x_replay, plain[0])
+    assert len(pats) == len(degs) and all(len(p) == nh + 1 for p in pats)
+    for a, b in zip(run(pats), plain):
+        assert torch.equal(a, b)
+    # first pass: x = 0, every row has the same pattern - one [1, h] row stands for all of them
+    first_row = [[t[:1] for t in pats[0]]] + pats[1:]
+    for a, b in zip(run(first_row), plain):
+        assert torch.equal(a, b)
+
+    # flip one active unit of degree 0 (it feeds every output but the first) in the last pass, whose outputs are final
+    row = int(torch.nonzero(pats[-1][0][:, 0])[0, 0])
+    flipped = [[t.clone() for t in p] for p in pats]
+    flipped[-1][0][row, 0] = False
+    _, _, (n_flip, _) = made_relu_patterns(Z, W, B, masks, degs, against=flipped)
+    assert n_flip == 1
+    got = run(flipped)
+    others = torch.arange(N) != row
+    for i in (0, 2):                                         # x and dz: row-local
+        assert torch.equal(got[i][others], plain[i][others])
+        assert not torch.equal(got[i][row], plain[i][row])
+    assert torch.equal(got[1][others], plain[1][others])
+
+    # the flow: MADE, reverse, MADE, reverse - patterns per MADE through iaf_forward and kgvae_encode's plumbing
+    h, n_flows = 10, 2
+    params = {k: v.double().requires_grad_(True) for k, v in O.init_params(30, h, 3, 2, 4, n_flows, seed=5).items()}
+    z0 = torch.randn(30, h, generator=gen, dtype=torch.float64)
+    z_p, lds_p, flp_p = O.iaf_forward(z0, params, n_flows)
+    (z_p.pow(2).sum() + flp_p).backward()
+    plain_grads = {k: v.grad.clone() for k, v in params.items() if v.grad is not None}
+    flow_pats, zc = [], z0
+    with torch.no_grad():
+        for ws, bs in O.flow_params(params, n_flows):
+            zc, pats_f, _ = made_relu_patterns(zc, ws, bs, O.made_masks(h, h, n_flows), O.made_degrees(h, h, n_flows))
+            flow_pats.append(pats_f)
+            zc = zc.flip(1)
+    assert torch.equal(zc, z_p.detach())
+    for v in params.values():
+        v.grad = None
+    z_q, lds_q, flp_q = O.iaf_forward(z0, params, n_flows, flow_pats)
+    (z_q.pow(2).sum() + flp_q).backward()
+    assert torch.equal(z_q, z_p) and torch.equal(lds_q, lds_p)
+    assert plain_grads.keys() == {k for k, v in params.items() if v.grad is not None}
+    for k, g in plain_grads.items():
+        assert torch.equal(params[k].grad, g), k
 
 
 def test_bdd_equals_dense_block_diagonal():

@@ -1,25 +1,13 @@
-// a3: RelGraphConv(regularizer="bdd") message passing in RELATION-MAJOR order.
-//
-// Per edge the layer needs the whole block-diagonal weight of the edge's relation: B*si*so
-// floats (10 KB for 5x5 blocks, 20 KB for 5x10) against a 2 KB source row.  Walking edges in
-// destination order (rgcn_bdd.cu, first version) re-reads those weights from L2 for every
-// edge - 5-10x the feature bytes.  Here edges are walked in (node tile, relation) order - the
-// etype-major record lists kg_graph_index / kg_graph_rel_tiled build - so that
-//   * a thread keeps ITS columns of W_r in REGISTERS for a whole run of edges (no per-edge weight
-//     traffic at all, not even shared memory), and
-//   * the rows that are reduced into (out[dst] forward, dx[src] backward) belong to one node tile
-//     sized to stay L2-resident, so the vector reductions never reach HBM and the only per-edge
-//     HBM traffic is the gathered row (forward: x[src]; backward: dagg[dst]).
-//
-//   forward   out[dst] += norm * blockdiag(W_r) x[src]          message accumulated with
-//   dX        dx[src]  += norm * blockdiag(W_r)^T dagg[dst]     128-bit vector reductions (RED.v4)
-//   dW        dW_r     += norm * x[src] (x) dagg[dst] blockwise registers, one flush per run
-//
-// A CTA takes 128 consecutive records (copied to shared memory once - no dependent index loads in
-// the loop) and splits into independent SLOTS of 4 or 8 warps, one edge per slot at a time; every
-// slot runs its own 4-deep cp.async ring of gathered rows and synchronises with a named barrier,
-// so there is no CTA-wide barrier in the loop.  dX and dW share one kernel (both need the gathered
-// dagg row).  Summation order across CTAs is not fixed: results are reproducible to fp32 rounding.
+// a3: RelGraphConv(regularizer="bdd") message passing over relation-sorted edge records
+// {src, dst, etype, norm} (kg_graph_index / kg_graph_rel_tiled), C entry points.  A call runs the
+// first kernel family that takes its block shape:
+//   1. block-owner kernels (rgcn_bdd_warp.cuh): 5x5 blocks (B % 4 == 0, B <= 128) and 5x10 blocks
+//      (B even, B <= 128), straight from the DGL-layout weight.  The only family for peer row
+//      blocks and for column chunks (the _cols entry points).
+//   2. register-tile kernels (rgcn_bdd_tile.cuh): blocks whose sides divide by 4, 5, 8, 10, 20, 25
+//      or 50, on the derived w_fwd / w_bwd layouts (kg_bdd_weight_layouts).  Backward is two
+//      launches: dX (the forward kernel on the transposed layout), then dW.
+//   3. the generic pair below: any shape whose relation weights fit in shared memory.
 #include "common.cuh"
 
 #include "rgcn_bdd_own.cuh"
@@ -30,287 +18,10 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int kChunk = 128;   // consecutive relation-sorted edges per CTA
-constexpr int kDepth = 4;     // gathered rows in flight per slot
 
 // hints (bit mask) of the C entry points: which gathered matrix is streamed from HBM (larger than
 // L2, every row used about once) and should not displace the L2-resident reduction tile
-constexpr int kHintStreamX = 1, kHintStreamD = 2;
-
-__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
-  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d)
-               : "memory");
-}
-__device__ __forceinline__ uint64_t l2_policy(bool evict_first) {
-  uint64_t pol;
-  if (evict_first) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  else asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void cp_async16(float* dst, const float* __restrict__ src, uint64_t pol) {
-  const uint32_t d = static_cast<uint32_t>(__cvta_generic_to_shared(dst));
-  asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"(d), "l"(src), "l"(pol)
-               : "memory");
-}
-__device__ __forceinline__ void async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-// named barrier of one slot; immediate ids so that the CTA reserves 1 + slots barriers, not all 16
-template <int NS>
-__device__ __forceinline__ void slot_barrier(int slot, int n) {
-  if (NS == 1) {
-    asm volatile("bar.sync 1, %0;" ::"r"(n) : "memory");
-    return;
-  }
-  if (NS == 2) {
-    if (slot == 0) asm volatile("bar.sync 1, %0;" ::"r"(n) : "memory");
-    else asm volatile("bar.sync 2, %0;" ::"r"(n) : "memory");
-    return;
-  }
-  switch (slot) {
-    case 0: asm volatile("bar.sync 1, %0;" ::"r"(n) : "memory"); break;
-    case 1: asm volatile("bar.sync 2, %0;" ::"r"(n) : "memory"); break;
-    case 2: asm volatile("bar.sync 3, %0;" ::"r"(n) : "memory"); break;
-    case 3: asm volatile("bar.sync 4, %0;" ::"r"(n) : "memory"); break;
-    case 4: asm volatile("bar.sync 5, %0;" ::"r"(n) : "memory"); break;
-    case 5: asm volatile("bar.sync 6, %0;" ::"r"(n) : "memory"); break;
-    case 6: asm volatile("bar.sync 7, %0;" ::"r"(n) : "memory"); break;
-    default: asm volatile("bar.sync 8, %0;" ::"r"(n) : "memory"); break;
-  }
-}
-
-// 4 consecutive output columns j0..j0+3 of  v (blockwise) times the per-thread weight registers:
-//   m[c] = sum_{i<K} v[((j0 + c) / F) * K + i] * w[i][c]
-// va / vb point at the blocks of columns j0 and j0+3 (the 4 columns touch at most 2 blocks); for
-// even F the column pairs (0,1) and (2,3) never straddle, for F % 4 == 0 nothing does.
-template <int K, int F>
-__device__ __forceinline__ float4 block_dot4(const float* va, const float* vb, const float4 (&w)[K], bool s1,
-                                             bool s2) {
-  float4 m = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-  for (int i = 0; i < K; ++i) {
-    const float xa = va[i];
-    if (F % 4 == 0) {
-      m.x = fmaf(xa, w[i].x, m.x);
-      m.y = fmaf(xa, w[i].y, m.y);
-      m.z = fmaf(xa, w[i].z, m.z);
-      m.w = fmaf(xa, w[i].w, m.w);
-    } else {
-      const float xb = vb[i];
-      m.x = fmaf(xa, w[i].x, m.x);
-      m.y = fmaf((F % 2 == 0 || s1) ? xa : xb, w[i].y, m.y);
-      m.z = fmaf((F % 2 != 0 && s2) ? xa : xb, w[i].z, m.z);
-      m.w = fmaf(xb, w[i].w, m.w);
-    }
-  }
-  return m;
-}
-
-__device__ __forceinline__ const float* row_ptr32(const float* base, int row, int width) {
-  return base + (size_t)(unsigned)row * (unsigned)width;      // one IMAD.WIDE.U32
-}
-
-// out[dst] += norm * blockdiag(W_etype) feat[src]; W layout [R][FI][B*FO]; out zero-filled by caller
-template <int FI, int FO, int NS>
-__global__ void __launch_bounds__(kThreads)
-bdd_rel_scatter_kernel(const float* __restrict__ feat, const int4* __restrict__ pack, int E,
-                       const float* __restrict__ wl, int B, int slot_t, int hints, float* __restrict__ out) {
-  extern __shared__ __align__(16) float sm[];
-  const int width = B * FO, in_w = B * FI;
-  int4* P_s = reinterpret_cast<int4*>(sm);    // [kChunk] {src, dst, etype, norm}
-  float* X_s = sm + 4 * kChunk;               // [slots][kDepth][in_w]
-  const int slots = NS == 8 ? kThreads / slot_t : NS;
-  const int slot = threadIdx.x / slot_t, st = threadIdx.x - slot * slot_t;
-  const int e0 = blockIdx.x * kChunk, n = min(E - e0, kChunk);
-  for (int i = threadIdx.x; i < n; i += kThreads) P_s[i] = __ldg(pack + e0 + i);
-  __syncthreads();
-  if (slot >= slots) return;
-  const uint64_t pol = l2_policy(hints & kHintStreamX);
-  const int n_my = (n - slot + slots - 1) / slots;      // this slot's edges: slot, slot + slots, ...
-  const int4* rec = P_s + slot;                         // record of edge k: rec[k * slots]
-  float* ring = X_s + slot * kDepth * in_w;
-  const bool copier = st < in_w / 4;                    // one 16-byte piece of the gathered row each
-  float* my_piece = ring + 4 * st;
-  const float* feat_piece = feat + 4 * st;
-
-  const bool active = st < width / 4;
-  const int j0 = active ? st * 4 : 0;
-  const int b0 = j0 / FO, b3 = (j0 + 3) / FO;
-  const bool s1 = (j0 + 1) / FO == b0, s2 = (j0 + 2) / FO == b0;
-  const float* xa = ring + b0 * FI;
-  const float* xb = ring + (FO % 2 == 0 && FO % 4 != 0 ? (j0 + 2) / FO : b3) * FI;
-  float* out_j = out + j0;
-  const float* wl_j = wl + j0;
-
-#pragma unroll
-  for (int k = 0; k < kDepth - 1; ++k) {                // prologue: rows 0 .. kDepth-2 in flight
-    if (k < n_my && copier) cp_async16(my_piece + k * in_w, row_ptr32(feat_piece, rec[k * slots].x, in_w), pol);
-    async_commit();                                     // one group per k, empty past the end
-  }
-
-  float4 w[FI];
-  int cur = -1;
-  const int4* rk = rec;                                 // record of the edge being processed
-  const int4* rn = rec + (kDepth - 1) * slots;          // record of the edge being prefetched
-  for (int k = 0; k < n_my; k += kDepth) {
-#pragma unroll
-    for (int u = 0; u < kDepth; ++u) {
-      if (k + u < n_my) {                               // uniform across the slot
-        async_wait<kDepth - 2>();                       // row k+u has landed (this thread's piece)
-        slot_barrier<NS>(slot, slot_t);                 // ... everybody's; row k+u-1 is consumed
-        if (k + u + kDepth - 1 < n_my && copier)        // refill the buffer row k+u-1 used
-          cp_async16(my_piece + ((u + kDepth - 1) % kDepth) * in_w, row_ptr32(feat_piece, rn->x, in_w), pol);
-        async_commit();
-        const int4 p = *rk;
-        rk += slots;
-        rn += slots;
-        if (active) {
-          if (p.z != cur) {                             // relation run starts: my 4 columns of W_r
-            cur = p.z;
-            const float* wr = row_ptr32(wl_j, cur, FI * width);
-#pragma unroll
-            for (int i = 0; i < FI; ++i) w[i] = __ldg(reinterpret_cast<const float4*>(wr + i * width));
-          }
-          const float nv = __int_as_float(p.w);
-          const float4 m = block_dot4<FI, FO>(xa + u * in_w, xb + u * in_w, w, s1, s2);
-          red_add_v4(const_cast<float*>(row_ptr32(out_j, p.y, width)), nv * m.x, nv * m.y, nv * m.z, nv * m.w);
-        }
-      }
-    }
-  }
-}
-
-// smallest divisor of SO that leaves at most 32 accumulators (SI * SO / OS) per thread
-__host__ __device__ constexpr int col_splits(int si, int so) {
-  for (int os = 1; os <= so; ++os)
-    if (so % os == 0 && si * so / os <= 32) return os;
-  return so;
-}
-
-// fused backward: dx[src] += norm * blockdiag(W_r)^T dagg[dst]   and
-//                 dW[r][b][i][o] += norm * x[src][b*SI+i] * dagg[dst][b*SO+o]
-// w_bwd layout [R][SO][B*SI]; dx, dW zero-filled by the caller; dx may be null.
-// Weight gradient: a thread owns one block b (or 1/OS of its output columns) and keeps the
-// SI x SO/OS outer-product accumulators in registers, flushed when the relation changes.
-// Input gradient: a thread owns 4 columns of dx and the matching columns of W_r^T in registers.
-template <int SI, int SO, int NS>
-__global__ void __launch_bounds__(kThreads)
-bdd_rel_backward_kernel(const float* __restrict__ x, const float* __restrict__ dagg,
-                        const int4* __restrict__ pack, int E, const float* __restrict__ w_bwd, int B,
-                        int slot_t, int hints, float* __restrict__ dx, float* __restrict__ dW) {
-  extern __shared__ __align__(16) float sm[];
-  constexpr int OS = col_splits(SI, SO);   // output-column splits per block: <= 32 accumulators per thread
-  constexpr int SOS = SO / OS;
-  const int in_w = B * SI, out_w = B * SO, KW = B * SI * SO, row_w = in_w + out_w;
-  int4* P_s = reinterpret_cast<int4*>(sm);    // [kChunk]
-  float* R_s = sm + 4 * kChunk;               // [slots][kDepth][in_w + out_w]: x row then dagg row
-  const int slots = NS == 8 ? kThreads / slot_t : NS;
-  const int slot = threadIdx.x / slot_t, st = threadIdx.x - slot * slot_t;
-  const int e0 = blockIdx.x * kChunk, n = min(E - e0, kChunk);
-  for (int i = threadIdx.x; i < n; i += kThreads) P_s[i] = __ldg(pack + e0 + i);
-  __syncthreads();
-  if (slot >= slots) return;
-  const uint64_t pol_x = l2_policy(hints & kHintStreamX), pol_d = l2_policy(hints & kHintStreamD);
-  const int n_my = (n - slot + slots - 1) / slots;
-  const int4* rec = P_s + slot;
-  float* ring = R_s + slot * kDepth * row_w;
-  // gathered pieces of this thread: one of the x row, up to two of the dagg row (out_w <= 2 * in_w)
-  const bool cx = st < in_w / 4, cd0 = st < out_w / 4, cd1 = st + slot_t < out_w / 4;
-  float* px = ring + 4 * st;
-  float* pd = ring + in_w + 4 * st;
-  const float* x_piece = x + 4 * st;
-  const float* d_piece = dagg + 4 * st;
-
-  auto gather = [&](const int4* r, int buf) {
-    const int4 p = *r;
-    if (cx) cp_async16(px + buf * row_w, row_ptr32(x_piece, p.x, in_w), pol_x);
-    const float* dr = row_ptr32(d_piece, p.y, out_w);
-    if (cd0) cp_async16(pd + buf * row_w, dr, pol_d);
-    if (cd1) cp_async16(pd + buf * row_w + 4 * slot_t, dr + 4 * slot_t, pol_d);
-  };
-#pragma unroll
-  for (int k = 0; k < kDepth - 1; ++k) {
-    if (k < n_my) gather(rec + k * slots, k);
-    async_commit();
-  }
-
-  // weight-gradient role
-  const bool wrole = st < B * OS;
-  const int wb = wrole ? st / OS : 0, oh = wrole ? st % OS : 0;
-  const float* xw = ring + wb * SI;
-  const float* dw_s = ring + in_w + wb * SO + oh * SOS;
-  float acc[SI][SOS];
-#pragma unroll
-  for (int i = 0; i < SI; ++i)
-#pragma unroll
-    for (int o = 0; o < SOS; ++o) acc[i][o] = 0.f;
-  // input-gradient role
-  const bool xrole = dx != nullptr && st < in_w / 4;
-  const int j0 = xrole ? st * 4 : 0;
-  const int b0 = j0 / SI, b3 = (j0 + 3) / SI;
-  const bool s1 = (j0 + 1) / SI == b0, s2 = (j0 + 2) / SI == b0;
-  const float* da = ring + in_w + b0 * SO;
-  const float* db = ring + in_w + (SI % 2 == 0 && SI % 4 != 0 ? (j0 + 2) / SI : b3) * SO;
-  float* dx_j = dx + j0;
-  const float* wt_j = w_bwd + j0;
-  float4 wt[SO];
-  int cur = -1;
-
-  auto flush = [&](int r) {
-    if (wrole) {
-      float* dst = dW + (size_t)r * KW + wb * SI * SO + oh * SOS;
-#pragma unroll
-      for (int i = 0; i < SI; ++i)
-#pragma unroll
-        for (int o = 0; o < SOS; ++o) {
-          atomicAdd(dst + i * SO + o, acc[i][o]);
-          acc[i][o] = 0.f;
-        }
-    }
-  };
-
-  const int4* rk = rec;
-  const int4* rn = rec + (kDepth - 1) * slots;
-  for (int k = 0; k < n_my; k += kDepth) {
-#pragma unroll
-    for (int u = 0; u < kDepth; ++u) {
-      if (k + u < n_my) {
-        async_wait<kDepth - 2>();
-        slot_barrier<NS>(slot, slot_t);
-        if (k + u + kDepth - 1 < n_my) gather(rn, (u + kDepth - 1) % kDepth);
-        async_commit();
-        const int4 p = *rk;
-        rk += slots;
-        rn += slots;
-        if (p.z != cur) {
-          if (cur >= 0) flush(cur);
-          cur = p.z;
-          if (xrole) {
-            const float* wr = row_ptr32(wt_j, cur, SO * in_w);
-#pragma unroll
-            for (int o = 0; o < SO; ++o) wt[o] = __ldg(reinterpret_cast<const float4*>(wr + o * in_w));
-          }
-        }
-        const float nv = __int_as_float(p.w);
-        if (wrole) {
-          float xv[SI], dv[SOS];
-#pragma unroll
-          for (int i = 0; i < SI; ++i) xv[i] = nv * xw[u * row_w + i];
-#pragma unroll
-          for (int o = 0; o < SOS; ++o) dv[o] = dw_s[u * row_w + o];
-#pragma unroll
-          for (int i = 0; i < SI; ++i)
-#pragma unroll
-            for (int o = 0; o < SOS; ++o) acc[i][o] = fmaf(xv[i], dv[o], acc[i][o]);
-        }
-        if (xrole) {
-          const float4 m = block_dot4<SO, SI>(da + u * row_w, db + u * row_w, wt, s1, s2);
-          red_add_v4(const_cast<float*>(row_ptr32(dx_j, p.x, in_w)), nv * m.x, nv * m.y, nv * m.z, nv * m.w);
-        }
-      }
-    }
-  }
-  if (cur >= 0) flush(cur);
-}
+constexpr int kHintStreamD = 2;
 
 // ------------------------------------------------------------------------------------------
 // any block shape: run-time FI/FO, scalar reductions, dW accumulated in shared memory
@@ -394,54 +105,9 @@ bdd_rel_backward_generic(const float* __restrict__ x, const float* __restrict__ 
     for (int k = threadIdx.x; k < KW; k += kThreads) atomicAdd(dW + (size_t)cur * KW + k, A_s[k]);
 }
 
-// slot = the threads that work on one edge together, rounded up to whole warps
-int slot_threads(int per_edge) { return (per_edge + 31) / 32 * 32; }
-
-template <int FI, int FO>
-int launch_scatter(const float* feat, const void* pack, int E, const float* wl, int B, int hints, float* out,
-                   cudaStream_t st) {
-  const int width = B * FO, in_w = B * FI;
-  const int slot_t = slot_threads(width / 4), slots = kThreads / slot_t;
-  const size_t smem = sizeof(float) * ((size_t)4 * kChunk + (size_t)slots * kDepth * in_w);
-  auto kern = slots == 1 ? bdd_rel_scatter_kernel<FI, FO, 1>
-              : slots == 2 ? bdd_rel_scatter_kernel<FI, FO, 2> : bdd_rel_scatter_kernel<FI, FO, 8>;
-  KG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<kg_div_up(E, kChunk), kThreads, smem, st>>>(feat, reinterpret_cast<const int4*>(pack), E, wl, B, slot_t,
-                                                     hints, out);
-  KG_LAUNCH_OK();
-  return KG_OK;
-}
-
-template <int SI, int SO>
-int launch_backward(const float* x, const float* dagg, const void* pack, int E, const float* w_bwd, int B,
-                    int hints, float* dx, float* dW, cudaStream_t st) {
-  const int in_w = B * SI, out_w = B * SO;
-  const int per_edge = B * col_splits(SI, SO) > in_w / 4 ? B * col_splits(SI, SO) : in_w / 4;
-  const int slot_t = slot_threads(per_edge), slots = kThreads / slot_t;
-  const size_t smem = sizeof(float) * ((size_t)4 * kChunk + (size_t)slots * kDepth * (in_w + out_w));
-  auto kern = slots == 1 ? bdd_rel_backward_kernel<SI, SO, 1>
-              : slots == 2 ? bdd_rel_backward_kernel<SI, SO, 2> : bdd_rel_backward_kernel<SI, SO, 8>;
-  KG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<kg_div_up(E, kChunk), kThreads, smem, st>>>(x, dagg, reinterpret_cast<const int4*>(pack), E, w_bwd, B,
-                                                     slot_t, hints, dx, dW);
-  KG_LAUNCH_OK();
-  return KG_OK;
-}
-
-bool fast_shape(int B, int si, int so) {
-  const bool known = (si == 5 && so == 5) || (si == 5 && so == 10) || (si == 10 && so == 10) ||
-                     (si == 4 && so == 4) || (si == 8 && so == 8);
-  // vector width 4 on both feature widths, one thread per 4 columns, one thread per (block, column split)
-  return known && (B * si) % 4 == 0 && (B * so) % 4 == 0 && (B * so) / 4 <= kThreads && (B * si) / 4 <= kThreads &&
-         B * col_splits(si, so) <= kThreads;
-}
-
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 }  // namespace
-
-#define KG_BDD_DISPATCH(FN, SI_, SO_, ...) \
-  if (si == SI_ && so == SO_) return FN<SI_, SO_>(__VA_ARGS__)
 
 // 1 when kg_bdd_rel_fwd / kg_bdd_rel_bwd need the derived layouts of kg_bdd_weight_layouts for this
 // shape, 0 when they read the DGL-layout weight directly (block-owner kernels, rgcn_bdd_own.cuh)
@@ -467,13 +133,6 @@ extern "C" int kg_bdd_rel_fwd(const float* x, const void* x_parts, int part_rows
   }
   KG_REQUIRE(x_parts == nullptr, "bdd rel fwd: peer row blocks need the 5x5 / 5x10 block-owner kernels");
   KG_REQUIRE(w_fwd != nullptr, "bdd rel fwd: this block shape needs the w_fwd layout (kg_bdd_weight_layouts)");
-  if (fast_shape(num_bases, si, so) && aligned16(x) && aligned16(w_fwd) && aligned16(agg)) {
-    KG_BDD_DISPATCH(launch_scatter, 5, 5, x, rel_pack, n_edges, w_fwd, num_bases, hints, agg, st);
-    KG_BDD_DISPATCH(launch_scatter, 5, 10, x, rel_pack, n_edges, w_fwd, num_bases, hints, agg, st);
-    KG_BDD_DISPATCH(launch_scatter, 10, 10, x, rel_pack, n_edges, w_fwd, num_bases, hints, agg, st);
-    KG_BDD_DISPATCH(launch_scatter, 4, 4, x, rel_pack, n_edges, w_fwd, num_bases, hints, agg, st);
-    KG_BDD_DISPATCH(launch_scatter, 8, 8, x, rel_pack, n_edges, w_fwd, num_bases, hints, agg, st);
-  }
   if (bddtile::eligible(num_bases, si, so) && aligned16(x) && aligned16(w_fwd) && aligned16(agg))
     return bddtile::launch_fwd(x, rel_pack, n_edges, w_fwd, si, so, num_bases, 0, agg, st);
   const size_t smem = sizeof(float) * ((size_t)si * num_bases * so + (size_t)num_bases * si);
@@ -509,13 +168,6 @@ extern "C" int kg_bdd_rel_bwd(const float* x, const void* x_parts, int part_rows
   }
   KG_REQUIRE(x_parts == nullptr, "bdd rel bwd: peer row blocks need the 5x5 / 5x10 block-owner kernels");
   KG_REQUIRE(w_bwd != nullptr, "bdd rel bwd: this block shape needs the w_bwd layout (kg_bdd_weight_layouts)");
-  if (fast_shape(num_bases, si, so) && aligned16(x) && aligned16(dagg) && aligned16(w_bwd) && aligned16(dx)) {
-    KG_BDD_DISPATCH(launch_backward, 5, 5, x, dagg, rel_pack, n_edges, w_bwd, num_bases, hints, dx, dweight, st);
-    KG_BDD_DISPATCH(launch_backward, 5, 10, x, dagg, rel_pack, n_edges, w_bwd, num_bases, hints, dx, dweight, st);
-    KG_BDD_DISPATCH(launch_backward, 10, 10, x, dagg, rel_pack, n_edges, w_bwd, num_bases, hints, dx, dweight, st);
-    KG_BDD_DISPATCH(launch_backward, 4, 4, x, dagg, rel_pack, n_edges, w_bwd, num_bases, hints, dx, dweight, st);
-    KG_BDD_DISPATCH(launch_backward, 8, 8, x, dagg, rel_pack, n_edges, w_bwd, num_bases, hints, dx, dweight, st);
-  }
   if (bddtile::eligible(num_bases, si, so) && aligned16(x) && aligned16(dagg) && aligned16(w_bwd) &&
       aligned16(dx) && aligned16(dweight)) {
     if (dx != nullptr) {

@@ -1,11 +1,28 @@
-// a3: RelGraphConv(regularizer="bdd") message passing for LARGER diagonal blocks (10x10 ... 50x100:
-// num_bases 10 .. 50 at h = 500; DGL RelGraphConv as constructed at kgvae/model.py:54-59 with a small
-// --n-bases, e.g. the WN18 shape where DGL clamps num_bases to the 36 directed relation types).
+// a3: RelGraphConv(regularizer="bdd") message passing with register tiles, for diagonal blocks from
+// 4x4 to 50x100 whose sides divide by 4, 5, 8, 10, 20, 25 or 50 (pick_tile): e.g. num_bases 10 .. 50
+// at h = 500 (DGL RelGraphConv as constructed at kgvae/model.py:54-59 with a small --n-bases, such as
+// the WN18 shape where DGL clamps num_bases to the 36 directed relation types).  The reference model's
+// 5x5 and 5x10 blocks run on the block-owner kernels (rgcn_bdd_warp.cuh) while they fit there.
 //
-// Same walk as rgcn_bdd_rel.cu - relation-major records, a CTA takes 128 consecutive edges, slots of
-// whole warps work on one edge at a time behind their own cp.async ring - but the register tiling is
-// two-dimensional so that a relation's WHOLE block-diagonal weight (B*si*so floats, up to 50 000)
-// stays in the registers of the threads of one slot while the relation lasts:
+// Edges are walked in RELATION-MAJOR order.  Per edge the layer needs the whole block-diagonal weight
+// of the edge's relation: B*si*so floats (10 KB for 5x5 blocks, 20 KB for 5x10) against a 2 KB source
+// row.  Walking edges in destination order (rgcn_bdd.cu, first version) re-reads those weights from L2
+// for every edge - 5-10x the feature bytes.  Here edges are walked in (node tile, relation) order - the
+// etype-major record lists kg_graph_index / kg_graph_rel_tiled build - so that
+//   * the threads of a slot keep the relation's weight in REGISTERS for a whole run of edges (no
+//     per-edge weight traffic at all, not even shared memory), and
+//   * the rows that are reduced into (out[dst] forward, dx[src] backward) belong to one node tile
+//     sized to stay L2-resident, so the vector reductions never reach HBM and the only per-edge
+//     HBM traffic is the gathered row (forward: x[src]; backward: dagg[dst]).
+//
+// A CTA takes 128 consecutive records (copied to shared memory once - no dependent index loads in
+// the loop) and splits into independent SLOTS of whole warps, one edge per slot at a time; every
+// slot runs its own 4-deep cp.async ring of gathered rows and synchronises with a named barrier, so
+// there is no CTA-wide barrier in the loop.  Summation order across CTAs is not fixed: results are
+// reproducible to fp32 rounding.
+//
+// The register tiling is two-dimensional so that a relation's WHOLE block-diagonal weight (B*si*so
+// floats, up to 50 000) stays in the registers of the threads of one slot while the relation lasts:
 //
 //   forward / dX   a thread owns CO consecutive output columns (inside one block) and KI of the
 //                  block's K input rows: w[KI][CO] registers, KI shared-memory broadcasts and
@@ -249,7 +266,7 @@ struct Tile {
 // widest column vector dividing `cols`, then the largest instantiated row count dividing `rows` with
 // at most 100 registers of tile and at most 512 threads per edge
 inline Tile pick_tile(int rows, int cols, int B) {
-  static const int kRows[] = {50, 25, 20, 10};
+  static const int kRows[] = {50, 25, 20, 10, 8, 5, 4};
   const int co = cols % 4 == 0 ? 4 : cols % 2 == 0 ? 2 : 1;
   for (int ki : kRows) {
     if (rows % ki != 0 || ki * co > 100) continue;
@@ -314,6 +331,15 @@ int launch_dw_t(const float* x, const float* dagg, const void* pack, int E, int 
 #define KG_TILE_CASE(FN, KI_, CO_, ...) \
   if (t.ki == KI_ && t.co == CO_) return FN<KI_, CO_>(__VA_ARGS__)
 #define KG_TILE_DISPATCH(FN, ...)        \
+  KG_TILE_CASE(FN, 4, 1, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 4, 2, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 4, 4, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 5, 1, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 5, 2, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 5, 4, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 8, 1, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 8, 2, __VA_ARGS__);   \
+  KG_TILE_CASE(FN, 8, 4, __VA_ARGS__);   \
   KG_TILE_CASE(FN, 10, 1, __VA_ARGS__);  \
   KG_TILE_CASE(FN, 10, 2, __VA_ARGS__);  \
   KG_TILE_CASE(FN, 10, 4, __VA_ARGS__);  \

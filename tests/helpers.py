@@ -32,6 +32,15 @@ def assert_close(a, b, rtol=RTOL, what=""):
     assert e <= rtol, f"{what}: relative error {e:.3e} > {rtol:.1e}"
 
 
+def kernels_run(fn):
+    """Names of the CUDA kernels ``fn`` launches (torch.profiler), joined by " | "."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    return " | ".join(e.name for e in prof.events())
+
+
 def at_golden_rows(gv, key, t):
     """The rows of ``t`` that golden case ``gv`` keeps of output ``key``: all of them, unless the case stores a
     seeded sample of the rows (``rows/<key>``) to stay small."""

@@ -21,7 +21,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import O, RTOL, assert_close, made_relu_patterns, rel_err
+from helpers import O, RTOL, assert_close, kernels_run, made_relu_patterns, rel_err
 
 import gcn_vae_b200 as K
 from gcn_vae_b200 import _lib as L
@@ -235,14 +235,6 @@ def test_gemm_tile_kernel_flow_shapes(M, N, K, ta, tb):
         _gemm_case(M, N, K, ta, tb, pad, (False, False, False, True, True), gen)     # masked accumulate
 
 
-def _kernels_run(fn):
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    return " | ".join(e.name for e in prof.events())
-
-
 @pytest.mark.parametrize("M,N,K,path", [(64, 64, 1000, "tile"), (64, 64, 1024, "tc"), (63, 500, 500, "tile"),
                                         (64, 500, 500, "tc"), (8, 500, 32, "small_m"), (9, 500, 32, "tile"),
                                         (8, 500, 31, "tile"), (1, 1000, 500, "small_m")])
@@ -258,7 +250,7 @@ def test_gemm_dispatch_boundaries(M, N, K, path):
         bias = torch.randn(N, generator=g)
         out = torch.empty(M, N, device=DEV)
         ad, bd, biasd = a.to(DEV), b.to(DEV), bias.to(DEV)
-        names = _kernels_run(lambda: ops.gemm(ad, bd, out, trans_a=bool(ta), trans_b=bool(tb), bias=biasd, relu=True))
+        names = kernels_run(lambda: ops.gemm(ad, bd, out, trans_a=bool(ta), trans_b=bool(tb), bias=biasd, relu=True))
         for p, k in kernel.items():       # demangled or mangled (gemm_kernelILb1E...) names
             ran = k in names or k.replace("<", "I") in names
             assert ran == (p == path), f"{M}x{N}x{K}: expected the {path} kernel, ran: {names}"

@@ -258,6 +258,7 @@ def test_graph_rel_tiled_order_integer_exact(n, e, r, tile, by_src):
 
 
 @pytest.mark.parametrize("B,si,so", [(100, 5, 5), (100, 5, 10), (50, 10, 10), (24, 4, 4), (16, 8, 8), (8, 5, 5),
+                                     (160, 5, 5), (10, 16, 16),
                                      # register-tile kernels (rgcn_bdd_tile.cuh): the WN18-shape blocks, odd
                                      # widths, K-split threads, 512-thread slots
                                      (25, 20, 20), (25, 20, 40), (50, 10, 20), (20, 25, 25), (20, 25, 50),

@@ -24,6 +24,8 @@ _SIGNATURES = {
     "kg_peer_free": (_I, [_P]),
     "kg_graph_build_workspace_bytes": (_Z, [_I]),
     "kg_graph_build": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
+    "kg_sample_relabel_workspace_bytes": (_Z, [_I]),
+    "kg_sample_relabel": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "kg_graph_index_workspace_bytes": (_Z, [_I]),
     "kg_graph_index": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "kg_embedding_fwd": (_I, [_P, _P, _I, _I, _P, _P]),
@@ -59,6 +61,8 @@ _SIGNATURES = {
     "kg_kl_mog_fwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P]),
     "kg_kl_mog_bwd": (_I, [_P, _P, _P, _P, _P, _P, _F, _I, _I, _I, _P, _P, _P, _P, _P]),
     "kg_kl_mog_bwd_fused": (_I, [_P, _P, _P, _P, _P, _P, _F, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
+    "kg_kl_mog_fwd_rows": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "kg_kl_mog_bwd_fused_rows": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "kg_iaf_update_fwd": (_I, [_P, _P, _P, _P, _I, _I, _P, _P, _P]),
     "kg_iaf_update_bwd": (_I, [_P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P]),
     "kg_reverse_columns": (_I, [_P, _I, _I, _P, _P]),
@@ -67,6 +71,7 @@ _SIGNATURES = {
     "kg_bce_logits_fwd": (_I, [_P, _P, _I, _P, _P, _P, _Z, _P]),
     "kg_sum_squares": (_I, [_P, _L, _P, _P, _Z, _P]),
     "kg_sum": (_I, [_P, _L, _P, _P, _Z, _P]),
+    "kg_sum_squares_rows": (_I, [_P, _I, _I, _P, _P, _P, _Z, _P]),
     "kg_triplet_index_workspace_bytes": (_Z, [_I]),
     "kg_triplet_index": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _Z, _P]),
     "kg_distmult_bce_workspace_bytes": (_Z, [_I]),
@@ -108,6 +113,7 @@ KERNELS_PER_CALL = {
     "kg_graph_build": 14, "kg_graph_index": 10, "kg_graph_rel_tiled": 5, "kg_triplet_index": 13, "kg_triplet_index_trailing": 18, "kg_distmult_bce_fwd": 5, "kg_distmult_bce_fwd_lead": 5, "kg_colsum": 2, "kg_act_dropout_bwd_colsum": 1,
     "kg_gemm_f32": 5,        # two operand preparations (2 kernels each) + the product (+ split-K finish): a lower bound
     "kg_gemm_prepare": 2,
+    "kg_sample_relabel": 7, "kg_kl_mog_fwd_rows": 2, "kg_sum_squares_rows": 2,
     "kg_kl_mog_fwd": 2, "kg_bce_logits_fwd": 2, "kg_sum_squares": 2, "kg_sum": 2, "kg_distmult_rank": 3, "kg_distmult_topk": 5,
 }
 launches = 0          # running count of kernels launched through this binding

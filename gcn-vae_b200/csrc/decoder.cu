@@ -82,7 +82,10 @@ __device__ __forceinline__ float block_sum(float v) {
 // mode 0: sum x; 1: sum x^2; 2: BCE-with-logits(x, y) and dscore = (sigmoid(x) - y) * inv_n
 __global__ void __launch_bounds__(kThreads)
 reduce_stage1(const float* __restrict__ x, const float* __restrict__ y, long long n, int mode,
-              float inv_n, float* __restrict__ dscore, float* __restrict__ partial) {
+              float inv_n, float* __restrict__ dscore, float* __restrict__ partial,
+              const int* __restrict__ n_rows = nullptr, int row_len = 0) {
+  // n_rows (device, may be NULL): only the first n_rows rows of row_len elements are read
+  if (n_rows != nullptr) n = min(n, (long long)__ldg(n_rows) * row_len);
   float s = 0.f;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
        i += (long long)gridDim.x * blockDim.x) {
@@ -114,7 +117,8 @@ extern "C" size_t kg_reduce_workspace_bytes(long long n) {
 }
 
 static int run_reduce(const float* x, const float* y, long long n, int mode, float scale, float inv_n,
-                      float* dscore, float* out, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+                      float* dscore, float* out, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                      const int* n_rows = nullptr, int row_len = 0) {
   if (workspace_bytes < sizeof(float) * kMaxPartials)
     return kg_fail(KG_ERR_WORKSPACE, "reduce: workspace too small");
   if (n == 0) {
@@ -123,7 +127,7 @@ static int run_reduce(const float* x, const float* y, long long n, int mode, flo
   }
   const int blocks = reduce_blocks(n);
   float* partial = reinterpret_cast<float*>(workspace);
-  reduce_stage1<<<blocks, kThreads, 0, st>>>(x, y, n, mode, inv_n, dscore, partial);
+  reduce_stage1<<<blocks, kThreads, 0, st>>>(x, y, n, mode, inv_n, dscore, partial, n_rows, row_len);
   KG_LAUNCH_OK();
   reduce_stage2<<<1, 32, 0, st>>>(partial, blocks, scale, out);
   KG_LAUNCH_OK();
@@ -141,6 +145,15 @@ extern "C" int kg_sum_squares(const float* x, long long n, float* out, void* wor
                               size_t workspace_bytes, void* stream) {
   KG_REQUIRE(n >= 0, "sum_squares: bad size");
   return run_reduce(x, nullptr, n, 1, 1.f, 0.f, nullptr, out, workspace, workspace_bytes, kg_stream(stream));
+}
+
+// sum of squares over the first n_valid (device int) rows of an [n_rows, h] matrix: the regulariser mean(z^2) of a
+// sampled subgraph padded to a fixed node budget (the grid is sized by n_rows; no host read of n_valid)
+extern "C" int kg_sum_squares_rows(const float* x, int n_rows, int h, const int32_t* n_valid, float* out,
+                                   void* workspace, size_t workspace_bytes, void* stream) {
+  KG_REQUIRE(n_rows >= 0 && h > 0 && n_valid != nullptr, "sum_squares_rows: bad arguments");
+  return run_reduce(x, nullptr, (long long)n_rows * h, 1, 1.f, 0.f, nullptr, out, workspace, workspace_bytes,
+                    kg_stream(stream), n_valid, h);
 }
 
 extern "C" int kg_sum(const float* x, long long n, float* out, void* workspace, size_t workspace_bytes,

@@ -399,3 +399,91 @@ extern "C" int kg_graph_build(const int32_t* src, const int32_t* rel, const int3
   return KG_OK;
 }
 
+// ------------------------------------------------------------------------------------------
+// relabelling of a sampled edge set with a fixed node budget (utils.SampledDeviceSampler)
+// np.unique((src, dst), return_inverse=True) of kgvae/utils.py:85-124, with every size fixed by B and cap so the
+// call can sit inside a CUDA-graph capture: the 2B endpoint ids are sorted with their slots, a head flag marks
+// the first of each run of equal ids, an inclusive scan of the flags numbers the runs, and one scatter writes
+// the labels back to the slots and each distinct id to node_id[label].  Rows n_valid .. cap-1 of node_id are
+// padding: row i looks up entity i (an id in range that is used at most once more, so the embedding backward's
+// per-element atomics never pile up on one row).
+// ------------------------------------------------------------------------------------------
+__global__ void relabel_keys(const int* __restrict__ picked, int B, int* __restrict__ keys, int* __restrict__ slots,
+                             int* __restrict__ rel) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B) return;
+  keys[i] = picked[3 * i];
+  keys[B + i] = picked[3 * i + 2];
+  slots[i] = i;
+  slots[B + i] = B + i;
+  rel[i] = picked[3 * i + 1];
+}
+
+__global__ void relabel_heads(const int* __restrict__ sorted, int M, int* __restrict__ flags) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= M) return;
+  flags[i] = (i == 0 || sorted[i] != sorted[i - 1]) ? 1 : 0;
+}
+
+__global__ void relabel_scatter(const int* __restrict__ sorted, const int* __restrict__ slots,
+                                const int* __restrict__ run, int B, int cap, int* __restrict__ node_id,
+                                int* __restrict__ src, int* __restrict__ dst, int* __restrict__ n_valid) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int M = 2 * B;
+  const int nv = run[M - 1];                          // number of distinct ids
+  if (i < M) {
+    const int label = run[i] - 1;
+    const int s = slots[i];
+    if (s < B) src[s] = label;
+    else dst[s - B] = label;
+    if ((i == 0 || sorted[i] != sorted[i - 1]) && label < cap) node_id[label] = sorted[i];
+  }
+  if (i < cap && i >= nv) node_id[i] = i;             // padding row i looks up entity i
+  // a caller that breaks cap >= distinct ids still gets n_valid <= cap: nothing drawn from [0, n_valid) can index past
+  // the node set (the ids past cap are dropped, their labels are not meaningful)
+  if (i == 0) n_valid[0] = nv < cap ? nv : cap;
+}
+
+static size_t relabel_cub_bytes(int M) {
+  size_t a = 0, b = 0;
+  cub::DeviceRadixSort::SortPairs((void*)nullptr, a, (int*)nullptr, (int*)nullptr, (int*)nullptr, (int*)nullptr, M);
+  cub::DeviceScan::InclusiveSum((void*)nullptr, b, (int*)nullptr, (int*)nullptr, M);
+  return kg_align_up((a > b ? a : b) + 256);
+}
+
+extern "C" size_t kg_sample_relabel_workspace_bytes(int n_picks) {
+  const int M = 2 * (n_picks > 0 ? n_picks : 1);
+  return 5 * kg_align_up((size_t)M * 4) + relabel_cub_bytes(M) + 1024;
+}
+
+extern "C" int kg_sample_relabel(const int32_t* picked, int n_picks, int num_nodes, int cap, int32_t* node_id,
+                                 int32_t* src, int32_t* rel, int32_t* dst, int32_t* n_valid, void* workspace,
+                                 size_t workspace_bytes, void* stream) {
+  KG_REQUIRE(n_picks > 0 && num_nodes > 0 && n_picks < (1 << 29), "sample_relabel: bad sizes");
+  KG_REQUIRE(cap > 0 && cap <= num_nodes && cap <= 2 * n_picks, "sample_relabel: need 0 < cap <= min(2B, num_nodes)");
+  cudaStream_t st = kg_stream(stream);
+  const int B = n_picks, M = 2 * B;
+  KgArena ws(workspace, workspace_bytes);
+  int* k_in = ws.take<int>(M);
+  int* k_out = ws.take<int>(M);
+  int* s_in = ws.take<int>(M);
+  int* s_out = ws.take<int>(M);
+  int* run = ws.take<int>(M);
+  size_t temp_bytes = relabel_cub_bytes(M);
+  void* temp = ws.take<char>(temp_bytes);
+  if (!k_in || !k_out || !s_in || !s_out || !run || !temp)
+    return kg_fail(KG_ERR_WORKSPACE, "sample_relabel: workspace too small");
+  relabel_keys<<<kg_div_up(B, kThreads), kThreads, 0, st>>>(picked, B, k_in, s_in, rel);
+  KG_LAUNCH_OK();
+  size_t tb = temp_bytes;
+  KG_CUDA(cub::DeviceRadixSort::SortPairs(temp, tb, k_in, k_out, s_in, s_out, M, 0, bits_for(num_nodes), st));
+  relabel_heads<<<kg_div_up(M, kThreads), kThreads, 0, st>>>(k_out, M, run);
+  KG_LAUNCH_OK();
+  tb = temp_bytes;
+  KG_CUDA(cub::DeviceScan::InclusiveSum(temp, tb, run, run, M, st));
+  relabel_scatter<<<kg_div_up(M > cap ? M : cap, kThreads), kThreads, 0, st>>>(k_out, s_out, run, B, cap, node_id, src,
+                                                                               dst, n_valid);
+  KG_LAUNCH_OK();
+  return KG_OK;
+}
+

@@ -87,10 +87,16 @@ __global__ void __launch_bounds__(128, 4)
 kl_mog_fwd_kernel(const float* __restrict__ z, const float* __restrict__ zm,
                   const float* __restrict__ zv, const float* __restrict__ z_pre,
                   const float* __restrict__ ws, int n, int h, int k, float* __restrict__ kl_rows,
-                  float* __restrict__ resp) {
+                  float* __restrict__ resp, const int* __restrict__ n_valid) {
   const int row0 = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * kKlWarpRows;
   const int lane = threadIdx.x & 31;
-  if (row0 >= n) return;
+  // n_valid (device, may be NULL): rows n_valid .. n-1 are padding - kl_rows = 0, nothing else is computed or written
+  const int n_rows = n;
+  if (n_valid != nullptr) n = min(__ldg(n_valid), n_rows);
+  if (row0 >= n) {
+    if (lane < kKlWarpRows && row0 + lane < n_rows) kl_rows[row0 + lane] = 0.f;
+    return;
+  }
   const float* inv2v = ws + (size_t)k * h;
   const float* lsq = ws + (size_t)2 * k * h;
   float a[kKlWarpRows], b[kKlWarpRows][KM], lsum[KM];
@@ -172,6 +178,8 @@ kl_mog_fwd_kernel(const float* __restrict__ z, const float* __restrict__ zm,
 #pragma unroll
       for (int i = 0; i < KM; ++i)
         if (i < k && lane == (i & 31)) resp[(size_t)row * k + i] = expf(b[q][i] - lse);
+    } else if (row < n_rows && lane == 0) {
+      kl_rows[row] = 0.f;
     }
   }
 }
@@ -185,14 +193,29 @@ kl_mog_bwd_kernel(const float* __restrict__ z, const float* __restrict__ zm,
                   const float* __restrict__ ws, const float* __restrict__ resp, float scale, int n,
                   int h, int k, const float* __restrict__ coefs, const float* __restrict__ add,
                   float* __restrict__ dz, float* __restrict__ dmean,
-                  float* __restrict__ dvar, float* __restrict__ dz_pre) {
+                  float* __restrict__ dvar, float* __restrict__ dz_pre, const int* __restrict__ n_valid) {
   const int d = blockIdx.y * blockDim.x + threadIdx.x;
   if (d >= h) return;
+  const int r0 = blockIdx.x * kKlRows;
+  int r1 = min(n, r0 + kKlRows);
+  if (n_valid != nullptr) {
+    // rows n_valid .. n-1 are padding: exact zeros in dz / dmean / dvar, nothing added to dz_pre.  The mean's 1/n is
+    // formed as the host forms it (a double quotient rounded to float), so valid rows match kg_kl_mog_bwd_fused bitwise
+    const int nv = min(__ldg(n_valid), n);
+    for (int row = max(r0, nv); row < r1; ++row) {
+      const size_t off = (size_t)row * h + d;
+      dz[off] = 0.f;
+      dmean[off] = 0.f;
+      dvar[off] = 0.f;
+    }
+    r1 = min(r1, nv);
+    if (r0 >= r1) return;
+    scale = (float)(1.0 / (double)nv);
+  }
   // fused form (kg_kl_mog_bwd_fused): the whole gradient of the loss head wrt z in one pass -
   //   dz = coefs[0] * dKL/dz + coefs[1] * add + coefs[2] * z     (add: dz of the DistMult term; z: the regulariser)
   const float c_add = coefs ? __ldg(coefs + 1) : 0.f, c_z = coefs ? __ldg(coefs + 2) : 0.f;
   if (coefs) scale *= __ldg(coefs);
-  const int r0 = blockIdx.x * kKlRows, r1 = min(n, r0 + kKlRows);
   // per mixture component i and column d, summed over the CTA's rows with r = resp[row, i], u = z - m_i:
   //   gpm = -sum r u / v_i          (gradient wrt the component mean)
   //   gpv = -sum r (u^2 / (2 v_i^2) - 1 / (2 v_i)) = -acc / (2 v_i)   with acc = sum ((r u / v_i) u - r)
@@ -238,9 +261,8 @@ kl_mog_bwd_kernel(const float* __restrict__ z, const float* __restrict__ zm,
     }
 }
 
-extern "C" int kg_kl_mog_fwd(const float* z, const float* z_mean, const float* z_var,
-                             const float* z_pre, int n, int h, int k, float* prior_ws, float* kl_rows,
-                             float* resp, void* stream) {
+static int kl_mog_fwd_impl(const float* z, const float* z_mean, const float* z_var, const float* z_pre, int n, int h,
+                           int k, const int* n_valid, float* prior_ws, float* kl_rows, float* resp, void* stream) {
   KG_REQUIRE(n >= 0 && h > 0 && k > 0 && k <= kMaxMix, "kl fwd: need 0 < k <= 16");
   cudaStream_t st = kg_stream(stream);
   prior_prepare_kernel<<<kg_div_up((long long)k * h, kThreads), kThreads, 0, st>>>(z_pre, k, h, prior_ws);
@@ -252,8 +274,10 @@ extern "C" int kg_kl_mog_fwd(const float* z, const float* z_mean, const float* z
                                    reinterpret_cast<uintptr_t>(prior_ws)) & 15) == 0;
 #define KG_KL_FWD(KM_)                                                                                          \
   do {                                                                                                          \
-    if (vec) kl_mog_fwd_kernel<KM_, 4><<<grid, 128, 0, st>>>(z, z_mean, z_var, z_pre, prior_ws, n, h, k, kl_rows, resp); \
-    else kl_mog_fwd_kernel<KM_, 1><<<grid, 128, 0, st>>>(z, z_mean, z_var, z_pre, prior_ws, n, h, k, kl_rows, resp);     \
+    if (vec) kl_mog_fwd_kernel<KM_, 4><<<grid, 128, 0, st>>>(z, z_mean, z_var, z_pre, prior_ws, n, h, k, kl_rows, resp, \
+                                                             n_valid);                                          \
+    else kl_mog_fwd_kernel<KM_, 1><<<grid, 128, 0, st>>>(z, z_mean, z_var, z_pre, prior_ws, n, h, k, kl_rows, resp,     \
+                                                         n_valid);                                              \
   } while (0)
   if (k <= 4) KG_KL_FWD(4);
   else if (k <= 8) KG_KL_FWD(8);
@@ -264,14 +288,30 @@ extern "C" int kg_kl_mog_fwd(const float* z, const float* z_mean, const float* z
   return KG_OK;
 }
 
+extern "C" int kg_kl_mog_fwd(const float* z, const float* z_mean, const float* z_var,
+                             const float* z_pre, int n, int h, int k, float* prior_ws, float* kl_rows,
+                             float* resp, void* stream) {
+  return kl_mog_fwd_impl(z, z_mean, z_var, z_pre, n, h, k, nullptr, prior_ws, kl_rows, resp, stream);
+}
+
+// The same over the first n_valid (device int) of n_rows rows: a sampled subgraph padded to a fixed node budget.
+// Rows past n_valid get kl_rows = 0 and cost no work; resp of those rows is not written.
+extern "C" int kg_kl_mog_fwd_rows(const float* z, const float* z_mean, const float* z_var, const float* z_pre,
+                                  int n_rows, int h, int k, const int32_t* n_valid, float* prior_ws, float* kl_rows,
+                                  float* resp, void* stream) {
+  KG_REQUIRE(n_valid != nullptr, "kl fwd rows: n_valid is required");
+  return kl_mog_fwd_impl(z, z_mean, z_var, z_pre, n_rows, h, k, n_valid, prior_ws, kl_rows, resp, stream);
+}
+
 // the per-thread mixture arrays are sized by the smallest instantiation that holds k (registers -> occupancy)
 static void launch_kl_bwd(dim3 grid, cudaStream_t st, const float* z, const float* zm, const float* zv, const float* z_pre,
                           const float* ws, const float* resp, float scale, int n, int h, int k, const float* coefs,
-                          const float* add, float* dz, float* dmean, float* dvar, float* dz_pre) {
-  if (k <= 4) kl_mog_bwd_kernel<4><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre);
-  else if (k <= 8) kl_mog_bwd_kernel<8><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre);
-  else if (k <= 12) kl_mog_bwd_kernel<12><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre);
-  else kl_mog_bwd_kernel<16><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre);
+                          const float* add, float* dz, float* dmean, float* dvar, float* dz_pre,
+                          const int* n_valid = nullptr) {
+  if (k <= 4) kl_mog_bwd_kernel<4><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre, n_valid);
+  else if (k <= 8) kl_mog_bwd_kernel<8><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre, n_valid);
+  else if (k <= 12) kl_mog_bwd_kernel<12><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre, n_valid);
+  else kl_mog_bwd_kernel<16><<<grid, 128, 0, st>>>(z, zm, zv, z_pre, ws, resp, scale, n, h, k, coefs, add, dz, dmean, dvar, dz_pre, n_valid);
 }
 
 extern "C" int kg_kl_mog_bwd(const float* z, const float* z_mean, const float* z_var,
@@ -301,6 +341,23 @@ extern "C" int kg_kl_mog_bwd_fused(const float* z, const float* z_mean, const fl
   dim3 grid(kg_div_up(n, kKlRows), kg_div_up(h, 128));
   launch_kl_bwd(grid, kg_stream(stream), z, z_mean, z_var, z_pre, prior_ws, resp, scale, n, h, k, coefs, add, dz, dmean,
                 dvar, dz_pre);
+  KG_LAUNCH_OK();
+  return KG_OK;
+}
+
+// kg_kl_mog_bwd_fused over the first n_valid (device int) of n_rows rows, scale = 1 / n_valid formed on the device:
+// rows n_valid .. n_rows-1 get exact zeros in dz, dmean and dvar and add nothing to dz_pre (CTAs wholly past
+// n_valid only write the zeros).
+extern "C" int kg_kl_mog_bwd_fused_rows(const float* z, const float* z_mean, const float* z_var, const float* z_pre,
+                                        const float* prior_ws, const float* resp, int n_rows, int h, int k,
+                                        const int32_t* n_valid, const float* coefs, const float* add, float* dz,
+                                        float* dmean, float* dvar, float* dz_pre, void* stream) {
+  KG_REQUIRE(n_rows >= 0 && h > 0 && k > 0 && k <= kMaxMix, "kl bwd rows: need 0 < k <= 16");
+  KG_REQUIRE(coefs != nullptr && n_valid != nullptr, "kl bwd rows: coefs and n_valid are required");
+  if (n_rows == 0) return KG_OK;
+  dim3 grid(kg_div_up(n_rows, kKlRows), kg_div_up(h, 128));
+  launch_kl_bwd(grid, kg_stream(stream), z, z_mean, z_var, z_pre, prior_ws, resp, 0.f, n_rows, h, k, coefs, add, dz,
+                dmean, dvar, dz_pre, n_valid);
   KG_LAUNCH_OK();
   return KG_OK;
 }

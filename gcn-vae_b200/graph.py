@@ -8,6 +8,10 @@ Call sites being served (reference): ``g = dgl.DGLGraph(); g.add_nodes(n); g.add
 Beyond that surface the graph owns the device-side edge orderings (ops.GraphIndex) that the
 message-passing kernels consume; they are built on first use for a given (etypes, norm) pair
 and reused by both RelGraphConv layers and their backward passes.
+
+``n_valid`` (default None): an int32 device tensor [1] when only the first n_valid nodes are real and the rest pad
+a sampled subgraph to a fixed node budget (utils.SampledDeviceSampler); the loss terms then average over the valid
+rows only.
 """
 import numpy as np
 import torch
@@ -41,6 +45,7 @@ class Graph:
         self.ndata, self.edata = {}, {}
         self._dev_edges = {}     # device -> (src int32, dst int32)
         self._index = None       # (key, ops.GraphIndex)
+        self.n_valid = None      # device int32 [1]: nodes past it are padding
 
     @classmethod
     def from_device_edges(cls, num_nodes, src, dst):
@@ -98,6 +103,7 @@ class Graph:
         g._n, g._src, g._dst = self._n, self._src, self._dst
         g.ndata, g.edata = dict(self.ndata), dict(self.edata)
         g._dev_edges, g._index = self._dev_edges, self._index
+        g.n_valid = self.n_valid
         return g
 
     def apply_edges(self, func):

@@ -71,26 +71,30 @@ class LinkPredict(nn.Module):
     def forward(self, g, h, r, norm):
         return self.encoder.forward(g, h, r, norm)
 
-    def regularization_loss(self, embedding):
-        return ops.MeanSquareFn.apply(embedding) + ops.MeanSquareFn.apply(self.w_relation)
+    def regularization_loss(self, embedding, n_valid=None):
+        """``n_valid``: the mean over the first n_valid rows of ``embedding`` only (a padded node set)."""
+        return ops.MeanSquareFn.apply(embedding, n_valid) + ops.MeanSquareFn.apply(self.w_relation)
 
     def get_loss(self, g, embed, triplets, labels):
-        """(loss, predict_loss, kl, mmd) as in link_predict.py:71-92."""
+        """(loss, predict_loss, kl, mmd) as in link_predict.py:71-92.  When ``g.n_valid`` is set (a sampled subgraph
+        padded to a fixed node budget) the per-node terms - regulariser, KL, MMD - cover the valid rows only and the
+        padding rows of z get exactly zero gradient."""
         if getattr(g, "partition", None) is not None:
             return self._get_loss_partitioned(g.partition, embed, triplets, labels)
         trip = ops.as_i32(triplets, embed.device)
         lab = torch.as_tensor(labels, dtype=torch.float32, device=embed.device)
         zero = lambda: torch.zeros(1, device=embed.device)
         enc = self.encoder
-        if isinstance(enc, KGVAE) and embed.requires_grad:
+        nv = getattr(g, "n_valid", None)
+        if isinstance(enc, KGVAE) and (embed.requires_grad or nv is not None):
             # pred + reg + KL in one autograd node: their gradients wrt z are combined in a single pass
             flp = enc.flow_log_prob if enc.n_flows > 0 else None
             head, predict_loss, reg_loss, kl_core = ops.LossHeadFn.apply(
                 embed, enc.z_mean, enc.z_sigma, enc.z_pre, self.w_relation, trip, lab, self._flow_shift(),
-                self.reg_param, self.kl_param)
+                self.reg_param, self.kl_param, nv)
             # the reference adds None here when n_flows == 0 and crashes (SURVEY F5); None -> 0
             kl = (kl_core if flp is None else kl_core + flp) if self.kl_param > 0 else zero()
-            mmd = enc.get_mmd(embed) if self.mmd_param > 0 else zero()
+            mmd = enc.get_mmd(embed, nv) if self.mmd_param > 0 else zero()
             loss = head
             if self.kl_param > 0 and flp is not None:
                 loss = loss + self.kl_param * flp
@@ -98,7 +102,7 @@ class LinkPredict(nn.Module):
                 loss = loss + self.mmd_param * mmd
             return loss, predict_loss, kl, mmd
         predict_loss = ops.DistMultBceFn.apply(embed, self.w_relation, trip, lab, self._flow_shift())
-        reg_loss = self.regularization_loss(embed)
+        reg_loss = self.regularization_loss(embed, nv)
         kl = self.encoder.get_kl(embed) if self.kl_param > 0 else zero()
         mmd = self.encoder.get_mmd(embed) if self.mmd_param > 0 else zero()
         loss = predict_loss + self.reg_param * reg_loss + self.kl_param * kl + self.mmd_param * mmd
@@ -158,9 +162,11 @@ class CapturedTrainStep:
     tensor (device; read it with ``float()`` when needed).
 
     ``sampler``: an object whose ``sample()`` returns that dict with fixed shapes using only stream-ordered device
-    work (``utils.FullBatchDeviceSampler``): the draw is then captured too and ``step()`` - no arguments - is the
-    whole iteration of the reference's loop (kgvae/link_predict.py:200-236): fresh negatives, fresh graph split,
-    edge index, forward, loss, backward, clip, Adam, in one replay (``example`` may be ``None``)."""
+    work (``utils.FullBatchDeviceSampler``, ``utils.SampledDeviceSampler``): the draw is then captured too and
+    ``step()`` - no arguments - is the whole iteration of the reference's loop (kgvae/link_predict.py:200-236): fresh
+    edge sample (SampledDeviceSampler), fresh negatives, fresh graph split, edge index, forward, loss, backward, clip,
+    Adam, in one replay (``example`` may be ``None``).  A sample with an ``n_valid`` entry (a node set padded to a
+    fixed budget) sets ``Graph.n_valid``, which keeps the padding rows out of the loss."""
 
     FIELDS = ("node_id", "src", "dst", "etype", "norm", "samples", "labels")
 
@@ -203,6 +209,7 @@ class CapturedTrainStep:
     def _eager(self):
         t = self.inputs if self.sampler is None else self.sampler.sample()
         g = self._Graph.from_device_edges(self.num_nodes, t["src"], t["dst"])
+        g.n_valid = t.get("n_valid")
         self.buckets.zero()
         embed = self.model(g, t["node_id"], t["etype"], t["norm"])
         loss, self.predict_loss, self.kl, self.mmd = self.model.get_loss(g, embed, t["samples"], t["labels"])
@@ -329,13 +336,20 @@ def main(args):
     captured = None
     if capture:
         # full-graph training: every iteration scores all training triples with fresh negatives on a fresh graph
-        # split - fixed shapes, so sampler + step are captured once and every iteration is one CUDA-graph replay
-        if args.graph_batch_size < len(train_data) or args.edge_sampler != "uniform":
-            raise RuntimeError("--capture-step needs full-batch uniform sampling: --graph-batch-size >= the number "
-                               f"of training triples ({len(train_data)}) and --edge-sampler uniform")
+        # split - fixed shapes, so sampler + step are captured once and every iteration is one CUDA-graph replay.
+        # Sampled subgraphs (--device-sampler): the node set is padded to a fixed budget, so their shapes are fixed too
+        full = args.graph_batch_size >= len(train_data)
+        sampled = getattr(args, "device_sampler", False)
+        if args.edge_sampler != "uniform" or not (full or sampled):
+            raise RuntimeError("--capture-step needs full-batch uniform sampling (--graph-batch-size >= the number of "
+                               f"training triples, {len(train_data)}) or --device-sampler, and --edge-sampler uniform")
         model.train()
         train_dev = torch.from_numpy(np.asarray(train_data)).to(device)
-        sampler = utils.FullBatchDeviceSampler(train_dev, num_rels, args.negative_sample, args.graph_split_size)
+        if full:
+            sampler = utils.FullBatchDeviceSampler(train_dev, num_rels, args.negative_sample, args.graph_split_size)
+        else:
+            sampler = utils.SampledDeviceSampler(train_dev, args.graph_batch_size, args.graph_split_size, num_rels,
+                                                 args.negative_sample)
         captured = CapturedTrainStep(model, optimizer, None, sampler.n, buckets=buckets, grad_norm=args.grad_norm,
                                      warmup=1, sampler=sampler)
         epoch += 1                       # the warm-up step that precedes the capture is a training step
@@ -428,7 +442,8 @@ def build_parser():
     p.add_argument("--load", type=bool, default=False)
     p.add_argument("--generate", type=bool, default=False)
     p.add_argument("--capture-step", action="store_true",
-                   help="(new) full-graph training (--graph-batch-size >= the number of training triples): negatives, "
+                   help="(new) full-graph training (--graph-batch-size >= the number of training triples), or sampled "
+                        "subgraphs with --device-sampler (nodes padded to min(2 B, entities)): edge sample, negatives, "
                         "graph split, edge index, forward, loss, backward, clipping and Adam are captured once into a "
                         "CUDA graph and every iteration is one replay; one warm-up iteration precedes the capture")
     p.add_argument("--device-sampler", action="store_true",

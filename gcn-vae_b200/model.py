@@ -88,7 +88,11 @@ class KGVAE(nn.Module):
                     log_det_sum = log_det if log_det_sum is None else log_det_sum + log_det
             self.log_det_sum = log_det_sum
             part = getattr(g, "partition", None)
-            if part is None:
+            n_valid = getattr(g, "n_valid", None)
+            if n_valid is not None:   # a padded node set: the mean over the valid rows
+                keep = ops.valid_rows(log_det_sum.shape[0], n_valid, log_det_sum.device)
+                self.flow_log_prob = torch.where(keep, log_det_sum, 0.0).sum() / n_valid.reshape(()).to(torch.float32)
+            elif part is None:
                 self.flow_log_prob = torch.mean(log_det_sum)
             else:                     # mean over ALL nodes: local sums, summed over the ranks
                 from . import parallel
@@ -109,16 +113,32 @@ class KGVAE(nn.Module):
         diff = x.unsqueeze(1) - y.unsqueeze(0)
         return torch.exp(-diff.pow(2).mean(2) / float(d))
 
-    def get_mmd(self, z):
+    def get_mmd(self, z, n_valid=None):
+        """``n_valid`` (device int32 [1], optional): only the first n_valid rows of z are nodes (a padded sampled
+        subgraph); the 200 posterior rows are then distinct valid rows drawn on the device (kept in ``mmd_rows``),
+        with no host read-back, so the term can be captured in a CUDA graph.  Like the unpadded path, which raises
+        through ``random.sample``, it needs 200 nodes: fewer than 200 rows raise, and a draw with n_valid < 200 makes
+        the term NaN (the host never reads n_valid, so the failure shows in the loss instead)."""
         m_mix, s_mix = utils.gaussian_parameters(self.z_pre, dim=1)
         num_sample = 200
         z_pri = utils.sample_gaussian(m_mix, s_mix, repeat=num_sample // self.k)
         if self.n_flows > 0:
             for flow in self.nf:
                 z_pri, _ = flow.forward(z_pri)
-        z_post = z[random.sample(range(z.shape[0]), num_sample)]
-        return (self.compute_kernel(z_pri, z_pri).mean() + self.compute_kernel(z_post, z_post).mean()
-                - 2 * self.compute_kernel(z_pri, z_post).mean())
+        if n_valid is None:
+            z_post = z[random.sample(range(z.shape[0]), num_sample)]
+        else:                         # the first 200 of a random order of the valid rows (padding keys sort last)
+            if z.shape[0] < num_sample:
+                raise ValueError(f"get_mmd: {z.shape[0]} node rows, the MMD term needs {num_sample}")
+            keys = torch.where(ops.valid_rows(z.shape[0], n_valid, z.device), torch.rand(z.shape[0], device=z.device),
+                               2.0)
+            self.mmd_rows = torch.argsort(keys)[:num_sample]
+            z_post = z[self.mmd_rows]
+        mmd = (self.compute_kernel(z_pri, z_pri).mean() + self.compute_kernel(z_post, z_post).mean()
+               - 2 * self.compute_kernel(z_pri, z_post).mean())
+        if n_valid is not None:       # padding rows entered z_post: no value rather than a wrong one
+            mmd = torch.where(n_valid.reshape(()) >= num_sample, mmd, float("nan"))
+        return mmd
 
     def get_mmd_partitioned(self, z_local, part):
         """get_mmd for destination-partitioned training (kgvae/model.py:89-102): the 200 posterior rows are

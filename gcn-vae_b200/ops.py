@@ -154,6 +154,29 @@ def graph_build(src, rel, dst, n_nodes, n_rels, node_major=False):
     return gi
 
 
+def sample_relabel(picked, num_nodes, cap):
+    """kg_sample_relabel: np.unique((src, dst), return_inverse=True) of B sampled triples (kgvae/utils.py:85-124)
+    with a fixed node budget ``cap``.  ``picked``: int32 [B, 3] on the device.  Returns (node_id int32 [cap],
+    src, rel, dst int32 [B], n_valid int32 [1]): rows 0 .. n_valid-1 of node_id are the distinct ids in ascending
+    order, row i >= n_valid holds entity i (padding).  No host read-back: capturable."""
+    picked = _c(picked)
+    dev = picked.device
+    B = int(picked.shape[0])
+    i32 = dict(dtype=torch.int32, device=dev)
+    node_id = torch.empty(int(cap), **i32)
+    src, rel, dst = (torch.empty(B, **i32) for _ in range(3))
+    n_valid = torch.empty(1, **i32)
+    ws = L.workspace(L.lib().kg_sample_relabel_workspace_bytes(B), dev)
+    L.call("kg_sample_relabel", L.i32(picked), B, int(num_nodes), int(cap), L.i32(node_id), L.i32(src), L.i32(rel),
+           L.i32(dst), L.i32(n_valid), L.ptr(ws), ws.numel(), L.stream())
+    return node_id, src, rel, dst, n_valid
+
+
+def valid_rows(n_rows, n_valid, device):
+    """bool [n_rows]: row < n_valid (device scalar), for masked means over a padded node set."""
+    return torch.arange(n_rows, device=device) < n_valid.reshape(())
+
+
 # ---------------------------------------------------------------------------------------------
 # dense GEMM helper
 # ---------------------------------------------------------------------------------------------
@@ -237,6 +260,15 @@ def act_dropout_bwd(g, out, mask, act, want_colsum=False):
     L.call("kg_act_dropout_bwd_colsum", L.f32(g), L.f32(out), L.f32(mask), act, rows, cols, L.f32(gpre), L.f32(dbias),
            L.ptr(ws), ws.numel(), L.stream())
     return gpre, dbias
+
+
+def _sum_squares_rows(x, n_valid):
+    """sum of squares over the first n_valid (device) rows of x [n, h] (kg_sum_squares_rows)."""
+    out = torch.empty((), dtype=torch.float32, device=x.device)
+    ws = L.workspace(L.lib().kg_reduce_workspace_bytes(x.numel()), x.device)
+    L.call("kg_sum_squares_rows", L.f32(x), x.shape[0], x.shape[1], L.i32(n_valid), L.f32(out), L.ptr(ws), ws.numel(),
+           L.stream())
+    return out
 
 
 def _reduce(name, x):
@@ -771,16 +803,26 @@ class LossHeadFn(torch.autograd.Function):
     gradient wrt z, scaled it by the upstream scalar with an elementwise multiply, and autograd added the three
     up: ten elementwise passes over 29 MB matrices.  Here backward forms the total in the KL backward pass
     (kg_kl_mog_bwd_fused): dz = c_kl dKL/dz + c_pred dz_pred + c_reg (2 / n h) z, coefficients on the device.
-    The scalar flow terms (flow_log_prob in the scores' shift and in the KL) stay with the caller."""
+    The scalar flow terms (flow_log_prob in the scores' shift and in the KL) stay with the caller.
+
+    ``n_valid`` (int32 device [1], optional): only the first n_valid rows of z are nodes, the rest pad a sampled
+    subgraph to a fixed node budget (utils.SampledDeviceSampler).  KL and regulariser are then means over the valid
+    rows (kg_kl_mog_fwd_rows, kg_sum_squares_rows, kg_kl_mog_bwd_fused_rows) and the gradient rows of the padding
+    are exactly zero; the triplets must only reference valid rows."""
 
     @staticmethod
-    def forward(ctx, z, z_mean, z_var, z_pre, w, triplets, labels, shift, reg_param, kl_param):
+    def forward(ctx, z, z_mean, z_var, z_pre, w, triplets, labels, shift, reg_param, kl_param, n_valid=None):
         z, w, labels = _c(z), _c(w), _c(labels)
         S, (n, h) = triplets.shape[0], z.shape
         dev = z.device
         out, dw, dz_pred = distmult_bce_pass(z, w, triplets, labels, shift, True)       # out: pred loss, sum of g
         pred = out[0].clone()
-        reg = _reduce("kg_sum_squares", z) / z.numel() + _reduce("kg_sum_squares", w) / w.numel()
+        if n_valid is None:
+            reg = _reduce("kg_sum_squares", z) / z.numel() + _reduce("kg_sum_squares", w) / w.numel()
+        else:
+            n_valid = _c(n_valid.reshape(1).to(torch.int32))
+            nv_f = n_valid.reshape(()).to(torch.float32)
+            reg = _sum_squares_rows(z, n_valid) / (nv_f * h) + _reduce("kg_sum_squares", w) / w.numel()
         use_kl = kl_param > 0 and z_mean is not None
         if use_kl:
             z_mean, z_var = _c(z_mean), _c(z_var)
@@ -789,15 +831,21 @@ class LossHeadFn(torch.autograd.Function):
             pws = torch.empty((3, k, h), dtype=torch.float32, device=dev)
             rows = torch.empty(n, dtype=torch.float32, device=dev)
             resp = torch.empty((n, k), dtype=torch.float32, device=dev)
-            L.call("kg_kl_mog_fwd", L.f32(z), L.f32(z_mean), L.f32(z_var), L.f32(zp), n, h, k, L.f32(pws),
-                   L.f32(rows), L.f32(resp), L.stream())
-            kl = _reduce("kg_sum", rows) / n
+            if n_valid is None:
+                L.call("kg_kl_mog_fwd", L.f32(z), L.f32(z_mean), L.f32(z_var), L.f32(zp), n, h, k, L.f32(pws),
+                       L.f32(rows), L.f32(resp), L.stream())
+                kl = _reduce("kg_sum", rows) / n
+            else:                                           # padding rows: kl_rows = 0
+                L.call("kg_kl_mog_fwd_rows", L.f32(z), L.f32(z_mean), L.f32(z_var), L.f32(zp), n, h, k,
+                       L.i32(n_valid), L.f32(pws), L.f32(rows), L.f32(resp), L.stream())
+                kl = _reduce("kg_sum", rows) / nv_f
             ctx.save_for_backward(z, w, dz_pred, dw, out, z_mean, z_var, zp, pws, resp)
             loss = pred + reg_param * reg + kl_param * kl
         else:
             kl = torch.zeros((), dtype=torch.float32, device=dev)
             ctx.save_for_backward(z, w, dz_pred, dw, out)
             loss = pred + reg_param * reg
+        ctx.n_valid = n_valid
         ctx.use_kl, ctx.reg_param, ctx.kl_param = use_kl, float(reg_param), float(kl_param)
         ctx.shift_shape = None if shift is None else shift.shape
         ctx.pre_shape = None if z_pre is None else z_pre.shape
@@ -814,22 +862,32 @@ class LossHeadFn(torch.autograd.Function):
         c_pred = g_loss + g_pred
         c_reg = g_loss * ctx.reg_param + g_reg
         c_kl = g_loss * ctx.kl_param + g_kl
+        nv = ctx.n_valid
+        # the regulariser's d mean(z^2) / dz = 2 z / (rows h): rows = n, or the valid rows of a padded node set
+        c_z = c_reg * (2.0 / z.numel()) if nv is None else c_reg * 2.0 / (nv.reshape(()).to(torch.float32) * h)
         dm = dv = dzp = None
         if ctx.use_kl:
             z_mean, z_var, zp, pws, resp = saved[5:]
             k = zp.shape[0] // 2
-            coefs = torch.stack([c_kl, c_pred, c_reg * (2.0 / z.numel())]).contiguous()
+            coefs = torch.stack([c_kl, c_pred, c_z]).contiguous()
             dz, dm, dv = (torch.empty_like(z) for _ in range(3))
             dzp = torch.zeros_like(zp)
-            L.call("kg_kl_mog_bwd_fused", L.f32(z), L.f32(z_mean), L.f32(z_var), L.f32(zp), L.f32(pws), L.f32(resp),
-                   1.0 / n, n, h, k, L.f32(coefs), L.f32(dz_pred), L.f32(dz), L.f32(dm), L.f32(dv), L.f32(dzp),
-                   L.stream(), tag="kg_kl_mog_bwd")
+            if nv is None:
+                L.call("kg_kl_mog_bwd_fused", L.f32(z), L.f32(z_mean), L.f32(z_var), L.f32(zp), L.f32(pws),
+                       L.f32(resp), 1.0 / n, n, h, k, L.f32(coefs), L.f32(dz_pred), L.f32(dz), L.f32(dm), L.f32(dv),
+                       L.f32(dzp), L.stream(), tag="kg_kl_mog_bwd")
+            else:                                           # padding rows: exact zeros, nothing into dz_pre
+                L.call("kg_kl_mog_bwd_fused_rows", L.f32(z), L.f32(z_mean), L.f32(z_var), L.f32(zp), L.f32(pws),
+                       L.f32(resp), n, h, k, L.i32(nv), L.f32(coefs), L.f32(dz_pred), L.f32(dz), L.f32(dm), L.f32(dv),
+                       L.f32(dzp), L.stream(), tag="kg_kl_mog_bwd")
             dzp = dzp.view(ctx.pre_shape)
         else:
-            dz = torch.addcmul(dz_pred * c_pred, z, c_reg * (2.0 / z.numel()))
+            dz = torch.addcmul(dz_pred * c_pred, z, c_z)
+            if nv is not None:                              # padding rows of z must not reach the encoder
+                dz = torch.where(valid_rows(n, nv, z.device).view(-1, 1), dz, 0.0)
         dwo = torch.addcmul(dw * c_pred, w, c_reg * (2.0 / w.numel()))
         dshift = (out[1] * c_pred).reshape(ctx.shift_shape) if ctx.shift_shape is not None else None
-        return dz, dm, dv, dzp, dwo, None, None, dshift, None, None
+        return dz, dm, dv, dzp, dwo, None, None, dshift, None, None, None
 
 
 class BceLogitsFn(torch.autograd.Function):
@@ -854,18 +912,27 @@ class BceLogitsFn(torch.autograd.Function):
 
 
 class MeanSquareFn(torch.autograd.Function):
-    """torch.mean(x.pow(2)) (kgvae/link_predict.py:68-69)."""
+    """torch.mean(x.pow(2)) (kgvae/link_predict.py:68-69).  ``n_valid`` (int32 device [1], optional): the mean over
+    the first n_valid rows of x [n, h] only (a node set padded to a fixed budget); padding rows get zero gradient."""
 
     @staticmethod
-    def forward(ctx, x):
+    def forward(ctx, x, n_valid=None):
         x = _c(x)
         ctx.save_for_backward(x)
-        return _reduce("kg_sum_squares", x) / x.numel()
+        if n_valid is None:
+            ctx.n_valid = None
+            return _reduce("kg_sum_squares", x) / x.numel()
+        ctx.n_valid = _c(n_valid.reshape(1).to(torch.int32))
+        return _sum_squares_rows(x, ctx.n_valid) / (ctx.n_valid.reshape(()).to(torch.float32) * x.shape[1])
 
     @staticmethod
     def backward(ctx, g):
         (x,) = ctx.saved_tensors
-        return x * (g * (2.0 / x.numel()))
+        nv = ctx.n_valid
+        if nv is None:
+            return x * (g * (2.0 / x.numel())), None
+        dx = x * (g * 2.0 / (nv.reshape(()).to(torch.float32) * x.shape[1]))
+        return torch.where(valid_rows(x.shape[0], nv, x.device).view(-1, 1), dx, 0.0), None
 
 
 # ---------------------------------------------------------------------------------------------

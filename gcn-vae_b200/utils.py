@@ -210,18 +210,80 @@ class FullBatchDeviceSampler:
         dev = self.src.device
         m = self.B * self.rate
         values = torch.randint(self.n, (m,), device=dev)
-        head = torch.rand(m, device=dev) > 0.5
-        neg = torch.stack([torch.where(head, values, self.neg_s), self.neg_r, torch.where(head, self.neg_o, values)], dim=1)
-        samples = torch.cat([self.pos, neg.to(torch.int32)])
-        keep = torch.argsort(torch.rand(self.B, device=dev))[:self.keep_n]       # a uniform random subset
-        s, r, d = self.src[keep], self.rel[keep], self.dst[keep]
-        src2, dst2 = torch.cat([s, d]), torch.cat([d, s])
-        etype = torch.cat([r, r + self.num_rels]).to(torch.int32)
-        deg = torch.zeros(self.n, dtype=torch.float32, device=dev).index_add_(
-            0, dst2, torch.ones(dst2.shape[0], dtype=torch.float32, device=dev))
-        norm = (1.0 / deg.clamp_(min=1.0))[dst2].view(-1, 1)
-        return {"node_id": self.node_id, "src": src2.to(torch.int32), "dst": dst2.to(torch.int32), "etype": etype,
-                "norm": norm, "samples": samples, "labels": self.labels}
+        samples = _with_negatives(self.pos, self.neg_s, self.neg_r, self.neg_o, values)
+        graph = _split_graph(self.src, self.rel, self.dst, self.keep_n, self.num_rels, self.n)
+        return {"node_id": self.node_id, **graph, "samples": samples, "labels": self.labels}
+
+
+def _with_negatives(pos, neg_s, neg_r, neg_o, values):
+    """The positives followed by their corruptions (kgvae/utils.py:158-171): one draw decides per negative whether
+    ``values`` replaces the subject (u > 0.5) or the object.  ``neg_*``: the positives' columns repeated."""
+    head = torch.rand(values.shape[0], device=values.device) > 0.5
+    neg = torch.stack([torch.where(head, values, neg_s), neg_r, torch.where(head, neg_o, values)], dim=1)
+    return torch.cat([pos, neg.to(torch.int32)])
+
+
+def _split_graph(src, rel, dst, keep_n, num_rels, n_nodes):
+    """A uniform random ``keep_n`` of the positives as graph structure, in both directions with reverse relation ids,
+    and 1 / in-degree norms over ``n_nodes`` nodes (0 edges: norm 1, unused) - kgvae/utils.py:115-150."""
+    dev = src.device
+    keep = torch.argsort(torch.rand(src.shape[0], device=dev))[:keep_n]       # a uniform random subset
+    s, r, d = src[keep], rel[keep], dst[keep]
+    src2, dst2 = torch.cat([s, d]), torch.cat([d, s])
+    etype = torch.cat([r, r + num_rels]).to(torch.int32)
+    deg = torch.zeros(n_nodes, dtype=torch.float32, device=dev).index_add_(
+        0, dst2, torch.ones(dst2.shape[0], dtype=torch.float32, device=dev))
+    norm = (1.0 / deg.clamp_(min=1.0))[dst2].view(-1, 1)
+    return {"src": src2.to(torch.int32), "dst": dst2.to(torch.int32), "etype": etype, "norm": norm}
+
+
+class SampledDeviceSampler:
+    """``generate_sampled_graph_and_labels_device`` with ``sample_size`` < len(triplets) in FIXED shapes, so that the
+    draw can be captured with the train step (``link_predict.CapturedTrainStep(..., sampler=...)``): every replay
+    then draws a fresh uniform edge sample, relabels it, draws negatives and a graph split, and trains on it.
+
+    Only the number of distinct entities among the B sampled triples varies from draw to draw.  The node set is
+    therefore padded to a fixed budget ``n = cap = min(2 B, distinct entities of the training triples)``, which no
+    draw can exceed: rows 0 .. n_valid-1 are the sampled nodes in ascending id order (as the eager device sampler
+    orders them), row i >= n_valid looks up entity i and has no edges.  ``n_valid`` stays on the device (int32
+    [1]); the model masks the padding out of every loss term through ``Graph.n_valid``.
+
+    ``sample()`` returns FullBatchDeviceSampler's dict plus ``n_valid``: ``node_id [cap, 1]`` (int32), ``src`` /
+    ``dst`` / ``etype [2 split B]`` (int32), ``norm [2 split B, 1]``, ``samples [B (1 + rate), 3]`` (int32),
+    ``labels``.  The B distinct picks are the first B of a sort of T uniforms (a uniform random B-subset), the
+    relabelling is kg_sample_relabel, negatives replace one end with floor(u n_valid).  Same procedure as the host
+    sampler (kgvae/utils.py:79-124,158-171), not numpy's random stream."""
+
+    def __init__(self, triplets, sample_size, split_size, num_rels, negative_rate):
+        if not triplets.is_cuda:
+            raise RuntimeError("SampledDeviceSampler needs the triples on a CUDA device (no CPU fallback)")
+        self.triplets = triplets.to(torch.int32).contiguous()
+        T = self.triplets.shape[0]
+        self.B = int(sample_size)
+        if not 0 < self.B <= T:
+            raise ValueError(f"SampledDeviceSampler: sample_size must be in 1 .. {T}, got {sample_size}")
+        ends = torch.cat([self.triplets[:, 0], self.triplets[:, 2]])
+        # the only host read-backs, once: the entity-id range and the number of distinct entities
+        self.num_nodes = int(ends.max()) + 1
+        self.n = min(2 * self.B, int(torch.unique(ends).numel()))
+        self.num_rels, self.rate = int(num_rels), int(negative_rate)
+        self.keep_n = int(self.B * split_size)
+        dev = self.triplets.device
+        self.labels = torch.zeros(self.B * (self.rate + 1), dtype=torch.float32, device=dev)
+        self.labels[:self.B] = 1
+        self.n_edges, self.n_samples = 2 * self.keep_n, self.B * (self.rate + 1)
+
+    def sample(self):
+        dev = self.triplets.device
+        picked = torch.argsort(torch.rand(self.triplets.shape[0], device=dev))[:self.B]
+        node_id, src, rel, dst, n_valid = ops.sample_relabel(self.triplets[picked], self.num_nodes, self.n)
+        pos = torch.stack([src, rel, dst], dim=1)
+        m = self.B * self.rate
+        # floor(u n_valid) with u in [0, 1) drawn in double: below n_valid for any n_valid < 2^24
+        values = (torch.rand(m, dtype=torch.float64, device=dev) * n_valid.to(torch.float64)).to(torch.int32)
+        samples = _with_negatives(pos, src.repeat(self.rate), rel.repeat(self.rate), dst.repeat(self.rate), values)
+        graph = _split_graph(src, rel, dst, self.keep_n, self.num_rels, self.n)
+        return {"node_id": node_id.view(-1, 1), **graph, "samples": samples, "labels": self.labels, "n_valid": n_valid}
 
 
 # --------------------------------------------------------------------------------------------

@@ -66,6 +66,19 @@ int kg_graph_build(const int32_t* src, const int32_t* rel, const int32_t* dst, i
                    int32_t* rel_ptr, void* rel_pack,
                    void* workspace, size_t workspace_bytes, void* stream);
 
+/* Relabelling of B sampled triples for a subgraph padded to a fixed node budget (kgvae/utils.py:85-124,
+ * np.unique((src, dst), return_inverse=True)), with every size fixed by B and cap - no host read-back, so the call
+ * can be captured in a CUDA graph.  picked [B, 3] int32 (s, r, o).  Outputs:
+ *   node_id [cap]: the n_valid distinct entity ids in ascending order, then padding rows i = n_valid .. cap-1
+ *                  holding entity i (in range; no id occurs more than twice)
+ *   src / dst [B]: relabelled end-points (0 .. n_valid-1), rel [B]: the relation column, n_valid [1]: device int.
+ * Needs 0 < cap <= min(2B, num_nodes) and cap >= the number of distinct ids (entity ids < num_nodes); with fewer
+ * rows than distinct ids, n_valid is clamped to cap and the ids past it are dropped. */
+size_t kg_sample_relabel_workspace_bytes(int n_picks);
+int kg_sample_relabel(const int32_t* picked, int n_picks, int num_nodes, int cap, int32_t* node_id,
+                      int32_t* src, int32_t* rel, int32_t* dst, int32_t* n_valid,
+                      void* workspace, size_t workspace_bytes, void* stream);
+
 /* Same index structures from an edge list the caller already ordered (the DGLGraph
  * surface: g.add_edges(src, dst) + etypes + per-edge norm, kgvae/utils.py:141-148).
  * Edges need not be sorted; the original edge order is kept as the tie-break so the
@@ -266,6 +279,17 @@ int kg_kl_mog_bwd_fused(const float* z, const float* z_mean, const float* z_var,
                         const float* prior_ws, const float* resp, float scale, int n, int h, int k,
                         const float* coefs, const float* add, float* dz, float* dmean, float* dvar,
                         float* dz_pre, void* stream);
+/* The forward and the fused backward over the first n_valid (DEVICE int) of n_rows rows - a sampled subgraph padded
+ * to a fixed node budget.  Valid rows compute exactly what kg_kl_mog_fwd / kg_kl_mog_bwd_fused compute on an
+ * [n_valid, h] input (bitwise); padding rows get kl_rows = 0 (resp unwritten) and exact zeros in dz, dmean and
+ * dvar, and add nothing to dz_pre.  The backward forms scale = 1 / n_valid itself. */
+int kg_kl_mog_fwd_rows(const float* z, const float* z_mean, const float* z_var, const float* z_pre,
+                       int n_rows, int h, int k, const int32_t* n_valid, float* prior_ws, float* kl_rows,
+                       float* resp, void* stream);
+int kg_kl_mog_bwd_fused_rows(const float* z, const float* z_mean, const float* z_var, const float* z_pre,
+                             const float* prior_ws, const float* resp, int n_rows, int h, int k,
+                             const int32_t* n_valid, const float* coefs, const float* add, float* dz,
+                             float* dmean, float* dvar, float* dz_pre, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * a6  IAF: element update of one MADE pass
@@ -304,6 +328,9 @@ int kg_sum_squares(const float* x, long long n, float* out, void* workspace, siz
                    void* stream);
 int kg_sum(const float* x, long long n, float* out, void* workspace, size_t workspace_bytes,
            void* stream);
+/* sum of squares over the first n_valid (device int) rows of x [n_rows, h] -> out[0]; workspace as kg_sum_squares */
+int kg_sum_squares_rows(const float* x, int n_rows, int h, const int32_t* n_valid, float* out, void* workspace,
+                        size_t workspace_bytes, void* stream);
 /* index structures, built once per batch of triplets (integer work, radix sort):
  *   rs_rec  [S]  int4 {a, r, b, t}: the triplets in (r, a) order - runs share w[r] and z[a].  DistMult
  *     is symmetric in its two entities, so {a, b} is {s, o} or, for batches of >= 2^14 triplets, {o, s}

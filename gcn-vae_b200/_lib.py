@@ -26,6 +26,8 @@ _SIGNATURES = {
     "kg_graph_build": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "kg_sample_relabel_workspace_bytes": (_Z, [_I]),
     "kg_sample_relabel": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
+    "kg_neighbor_sample_plan": (_I, [_I, _I, _I, _P, _P]),
+    "kg_neighbor_sample": (_I, [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _Z, _P]),
     "kg_graph_index_workspace_bytes": (_Z, [_I]),
     "kg_graph_index": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "kg_embedding_fwd": (_I, [_P, _P, _I, _I, _P, _P]),
@@ -114,6 +116,7 @@ KERNELS_PER_CALL = {
     "kg_gemm_f32": 5,        # two operand preparations (2 kernels each) + the product (+ split-K finish): a lower bound
     "kg_gemm_prepare": 2,
     "kg_sample_relabel": 7, "kg_kl_mog_fwd_rows": 2, "kg_sum_squares_rows": 2,
+    "kg_neighbor_sample_plan": 0, "kg_neighbor_sample": 1,
     "kg_kl_mog_fwd": 2, "kg_bce_logits_fwd": 2, "kg_sum_squares": 2, "kg_sum": 2, "kg_distmult_rank": 3, "kg_distmult_topk": 5,
 }
 launches = 0          # running count of kernels launched through this binding

@@ -166,7 +166,9 @@ class CapturedTrainStep:
     ``step()`` - no arguments - is the whole iteration of the reference's loop (kgvae/link_predict.py:200-236): fresh
     edge sample (SampledDeviceSampler), fresh negatives, fresh graph split, edge index, forward, loss, backward, clip,
     Adam, in one replay (``example`` may be ``None``).  A sample with an ``n_valid`` entry (a node set padded to a
-    fixed budget) sets ``Graph.n_valid``, which keeps the padding rows out of the loss."""
+    fixed budget) sets ``Graph.n_valid``, which keeps the padding rows out of the loss.  A sampler with a
+    ``before_replay()`` method has it called before every replay (the neighbourhood sampler refills its bank of edge
+    samples there)."""
 
     FIELDS = ("node_id", "src", "dst", "etype", "norm", "samples", "labels")
 
@@ -237,6 +239,9 @@ class CapturedTrainStep:
     def step(self, **tensors):
         if tensors:
             self.load(**tensors)
+        before = getattr(self.sampler, "before_replay", None)
+        if before is not None:            # e.g. a bank of edge samples that refills between replays
+            before()
         self.graph.replay()
         return self.loss
 
@@ -334,22 +339,26 @@ def main(args):
 
     train_dev = None
     captured = None
+    bank = None                          # eager --device-sampler --edge-sampler neighbor: a bank of edge samples
     if capture:
         # full-graph training: every iteration scores all training triples with fresh negatives on a fresh graph
         # split - fixed shapes, so sampler + step are captured once and every iteration is one CUDA-graph replay.
         # Sampled subgraphs (--device-sampler): the node set is padded to a fixed budget, so their shapes are fixed too
+        # Both edge samplers select every triple when B >= T, so FullBatchDeviceSampler serves both there
         full = args.graph_batch_size >= len(train_data)
         sampled = getattr(args, "device_sampler", False)
-        if args.edge_sampler != "uniform" or not (full or sampled):
-            raise RuntimeError("--capture-step needs full-batch uniform sampling (--graph-batch-size >= the number of "
-                               f"training triples, {len(train_data)}) or --device-sampler, and --edge-sampler uniform")
+        if args.edge_sampler not in ("uniform", "neighbor"):
+            raise ValueError("Sampler type must be either 'uniform' or 'neighbor'.")
+        if not (full or sampled):
+            raise RuntimeError("--capture-step needs full-batch sampling (--graph-batch-size >= the number of "
+                               f"training triples, {len(train_data)}) or --device-sampler")
         model.train()
         train_dev = torch.from_numpy(np.asarray(train_data)).to(device)
         if full:
             sampler = utils.FullBatchDeviceSampler(train_dev, num_rels, args.negative_sample, args.graph_split_size)
         else:
             sampler = utils.SampledDeviceSampler(train_dev, args.graph_batch_size, args.graph_split_size, num_rels,
-                                                 args.negative_sample)
+                                                 args.negative_sample, edge_sampler=args.edge_sampler)
         captured = CapturedTrainStep(model, optimizer, None, sampler.n, buckets=buckets, grad_norm=args.grad_norm,
                                      warmup=1, sampler=sampler)
         epoch += 1                       # the warm-up step that precedes the capture is a training step
@@ -370,12 +379,18 @@ def main(args):
             if epoch >= args.n_epochs:
                 break
             continue
-        if getattr(args, "device_sampler", False) and args.edge_sampler == "uniform":
+        if getattr(args, "device_sampler", False) and args.edge_sampler in ("uniform", "neighbor"):
             # opt-in: the same sampling procedure drawn on the GPU (not numpy's random stream)
             if train_dev is None:
                 train_dev = torch.from_numpy(np.asarray(train_data)).to(device)
+            picked = None
+            if args.edge_sampler == "neighbor" and args.graph_batch_size < len(train_data):
+                if bank is None:
+                    bank = utils.NeighborEdgeBank(train_dev, num_nodes, args.graph_batch_size)
+                picked = bank.next()
             g, node_id, edge_type, edge_norm, batch, labels = utils.generate_sampled_graph_and_labels_device(
-                train_dev, args.graph_batch_size, args.graph_split_size, num_rels, args.negative_sample)
+                train_dev, args.graph_batch_size, args.graph_split_size, num_rels, args.negative_sample,
+                picked=picked)
         else:
             g, node_id, edge_type, node_norm, batch, labels = utils.generate_sampled_graph_and_labels(
                 train_data, args.graph_batch_size, args.graph_split_size, num_rels, adj_list, degrees,
@@ -447,8 +462,9 @@ def build_parser():
                         "graph split, edge index, forward, loss, backward, clipping and Adam are captured once into a "
                         "CUDA graph and every iteration is one replay; one warm-up iteration precedes the capture")
     p.add_argument("--device-sampler", action="store_true",
-                   help="(new) draw the uniform edge sample, the negatives and the graph split on the GPU; same "
-                        "procedure as the reference's host sampler, not its numpy random stream")
+                   help="(new) draw the edge sample (--edge-sampler uniform or neighbor), the negatives and the "
+                        "graph split on the GPU; same procedure as the reference's host sampler, not its numpy random "
+                        "stream.  The neighbour sampler draws a bank of samples per kernel launch")
     return p
 
 

@@ -4,6 +4,7 @@ Each Function is one fused operator of the link-prediction path and names the re
 code it replaces.  All tensors are CUDA, fp32 / int32, contiguous; PyTorch supplies device
 memory, the stream and autograd bookkeeping only.
 """
+import ctypes
 import os
 
 import torch
@@ -170,6 +171,51 @@ def sample_relabel(picked, num_nodes, cap):
     L.call("kg_sample_relabel", L.i32(picked), B, int(num_nodes), int(cap), L.i32(node_id), L.i32(src), L.i32(rel),
            L.i32(dst), L.i32(n_valid), L.ptr(ws), ws.numel(), L.stream())
     return node_id, src, rel, dst, n_valid
+
+
+NEIGHBOR_WORDS, NEIGHBOR_TRIES = 8, 6         # KG_NEIGHBOR_WORDS / KG_NEIGHBOR_TRIES of include/kgvae_b200.h
+
+
+def neighbor_adjacency(triplets, num_nodes):
+    """The adjacency lists of utils.get_adj_and_degrees as a device CSR, built by one stable sort of the 2T ends:
+    ``adj_ptr`` int32 [N+1] and ``adj`` int32 [2T, 2] rows (edge id, other end), per entity in ascending edge id with
+    the subject end first for a self-loop.  ``triplets``: int tensor [T, 3] on the device."""
+    tri = _c(triplets).long()
+    ends = tri[:, [0, 2]].reshape(-1)                   # s0, o0, s1, o1, ...: edge order, subject end first
+    order = torch.sort(ends, stable=True).indices
+    other = tri[:, [2, 0]].reshape(-1)[order]
+    adj = torch.stack([order // 2, other], dim=1).to(torch.int32).contiguous()
+    adj_ptr = torch.zeros(int(num_nodes) + 1, dtype=torch.int32, device=tri.device)
+    adj_ptr[1:] = torch.cumsum(torch.bincount(ends, minlength=int(num_nodes)), 0)
+    return adj_ptr, adj
+
+
+def neighbor_sample_plan(num_nodes, n_triples, sample_size):
+    """(samples drawn per launch, workspace bytes) of kg_neighbor_sample on the current device."""
+    k, ws = ctypes.c_int(), ctypes.c_size_t()
+    L.call("kg_neighbor_sample_plan", int(num_nodes), int(n_triples), int(sample_size), ctypes.byref(k),
+           ctypes.byref(ws))
+    return k.value, ws.value
+
+
+def neighbor_sample(adj_ptr, adj, num_nodes, sample_size, words, out=None, fallbacks=None, workspace=None):
+    """kg_neighbor_sample: one neighbourhood-expansion sample (kgvae/utils.py:33-76) of ``sample_size`` distinct
+    triples per row of ``words`` (int32 [K, B, NEIGHBOR_WORDS], read as uniform 32-bit words).  Returns picks int32
+    [K, B] (edge ids).  ``fallbacks``: optional int32 [K] that receives, per sample, the picks that needed the scan
+    over unpicked entries.  Same procedure as the host sampler, not numpy's random stream; tests/neighbor_mirror.py is
+    its specification.  No host read-back: capturable."""
+    words = _c(words)
+    K, B = int(words.shape[0]), int(sample_size)
+    if words.shape[1:] != (B, NEIGHBOR_WORDS):
+        raise ValueError(f"neighbor_sample: words must be [K, {B}, {NEIGHBOR_WORDS}], got {tuple(words.shape)}")
+    dev = words.device
+    if out is None:
+        out = torch.empty(K, B, dtype=torch.int32, device=dev)
+    if workspace is None:
+        workspace = L.workspace(neighbor_sample_plan(num_nodes, adj.shape[0] // 2, B)[1], dev)
+    L.call("kg_neighbor_sample", L.i32(adj_ptr), L.i32(adj), int(num_nodes), int(adj.shape[0]) // 2, B, K,
+           L.i32(words), L.i32(out), L.i32(fallbacks), L.ptr(workspace), workspace.numel(), L.stream())
+    return out
 
 
 def valid_rows(n_rows, n_valid, device):

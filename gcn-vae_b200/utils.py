@@ -133,7 +133,7 @@ def generate_sampled_graph_and_labels(triplets, sample_size, split_size, num_rel
 
 
 def generate_sampled_graph_and_labels_device(triplets, sample_size, split_size, num_rels, negative_rate,
-                                             generator=None):
+                                             generator=None, picked=None):
     """Opt-in DEVICE form of ``generate_sampled_graph_and_labels`` with the uniform edge sampler
     (kgvae/utils.py:79-124,158-171): ``sample_size`` training triples without replacement, nodes
     relabelled to 0..n-1 in ascending id order, ``negative_rate`` corruptions per positive (subject
@@ -143,7 +143,9 @@ def generate_sampled_graph_and_labels_device(triplets, sample_size, split_size, 
     Everything stays on the GPU (torch's device generator + ``kg_graph_build``), so the step needs
     neither the host sampler nor the ~50 MB of host -> device copies.  The draws follow the same
     procedure but NOT numpy's random stream: use the host function when sampled indices must match
-    the reference bit for bit.  ``triplets``: int tensor [T, 3] on the device.
+    the reference bit for bit.  ``triplets``: int tensor [T, 3] on the device.  ``picked``: optional precomputed
+    edge sample (int tensor [sample_size] of distinct triple ids, e.g. ``NeighborEdgeBank.next()`` for the
+    neighbourhood sampler) used instead of the uniform draw.
 
     Returns (g, node_id [n, 1] int64, edge_type int32 [E], edge_norm f32 [E, 1], samples int32
     [S, 3], labels f32 [S]) - the arguments of ``model(g, node_id, edge_type, edge_norm)`` and
@@ -152,8 +154,9 @@ def generate_sampled_graph_and_labels_device(triplets, sample_size, split_size, 
         raise RuntimeError("generate_sampled_graph_and_labels_device needs the triples on a CUDA device")
     dev = triplets.device
     B, rate = int(sample_size), int(negative_rate)
-    picked = torch.randperm(triplets.shape[0], device=dev, generator=generator)[:B]
-    tri = triplets[picked].long()
+    if picked is None:
+        picked = torch.randperm(triplets.shape[0], device=dev, generator=generator)[:B]
+    tri = triplets[picked.long()].long()
     uniq_v, inv = torch.unique(torch.cat([tri[:, 0], tri[:, 2]]), return_inverse=True)
     n = int(uniq_v.numel())
     src, rel, dst = inv[:B], tri[:, 1], inv[B:]
@@ -237,6 +240,61 @@ def _split_graph(src, rel, dst, keep_n, num_rels, n_nodes):
     return {"src": src2.to(torch.int32), "dst": dst2.to(torch.int32), "etype": etype, "norm": norm}
 
 
+class NeighborEdgeBank:
+    """Neighbourhood-expansion edge samples (kgvae/utils.py:33-76, ``--edge-sampler neighbor``) drawn on the GPU a
+    bank at a time.  The picks of one sample are sequential, but samples are independent of each other and of the
+    model, so one ``kg_neighbor_sample`` launch draws K samples (K = what one wave of the device holds, chosen by the
+    library) into a persistent ``bank [K, B]`` and the training steps consume it one row at a time.
+
+    ``next()`` returns ``bank[cursor]`` and advances the device ``cursor`` with stream-ordered device ops, so it can
+    be captured in a CUDA graph.  The host keeps ``consumed``, the number of rows taken since the last refill, equal
+    to the device cursor: outside a capture ``next()`` counts its row itself (refilling first when the bank is used
+    up); a captured ``next()`` runs at every replay, and the caller calls ``before_replay()`` before each one, which
+    counts the row and refills eagerly between replays once all K rows are consumed.
+
+    ``refill()`` draws K x B x 8 uniform 32-bit words with torch's device generator and launches the kernel.  Same
+    procedure as the host sampler up to the 2^-32 granularity of the integer mapping, not numpy's random stream."""
+
+    def __init__(self, triplets, num_nodes, sample_size):
+        if not triplets.is_cuda:
+            raise RuntimeError("NeighborEdgeBank needs the triples on a CUDA device (no CPU fallback)")
+        dev = triplets.device
+        self.num_nodes, self.n_triples, self.B = int(num_nodes), int(triplets.shape[0]), int(sample_size)
+        self.adj_ptr, self.adj = ops.neighbor_adjacency(triplets, self.num_nodes)
+        self.K, ws = ops.neighbor_sample_plan(self.num_nodes, self.n_triples, self.B)
+        self.workspace = torch.empty(max(ws, 16), dtype=torch.uint8, device=dev)
+        self.words = torch.empty(self.K, self.B, ops.NEIGHBOR_WORDS, dtype=torch.int32, device=dev)
+        self.bank = torch.empty(self.K, self.B, dtype=torch.int32, device=dev)
+        self.cursor = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.consumed = self.K                   # empty: the first next() refills
+        self.refills = 0
+
+    def refill(self):
+        self.words.random_(-2 ** 31, 2 ** 31)
+        ops.neighbor_sample(self.adj_ptr, self.adj, self.num_nodes, self.B, self.words, out=self.bank,
+                            workspace=self.workspace)
+        self.cursor.zero_()
+        self.consumed = 0
+        self.refills += 1
+
+    def next(self):
+        """int32 [B]: the next row of the bank."""
+        if not torch.cuda.is_current_stream_capturing():
+            if self.consumed >= self.K:
+                self.refill()
+            self.consumed += 1
+        # the remainder only guards the gather; before_replay() keeps the cursor below K
+        row = self.bank.index_select(0, torch.remainder(self.cursor, self.K)).view(-1)
+        self.cursor.add_(1)
+        return row
+
+    def before_replay(self):
+        """Call before each replay of a graph that captured one ``next()``."""
+        if self.consumed >= self.K:
+            self.refill()
+        self.consumed += 1
+
+
 class SampledDeviceSampler:
     """``generate_sampled_graph_and_labels_device`` with ``sample_size`` < len(triplets) in FIXED shapes, so that the
     draw can be captured with the train step (``link_predict.CapturedTrainStep(..., sampler=...)``): every replay
@@ -252,9 +310,13 @@ class SampledDeviceSampler:
     ``dst`` / ``etype [2 split B]`` (int32), ``norm [2 split B, 1]``, ``samples [B (1 + rate), 3]`` (int32),
     ``labels``.  The B distinct picks are the first B of a sort of T uniforms (a uniform random B-subset), the
     relabelling is kg_sample_relabel, negatives replace one end with floor(u n_valid).  Same procedure as the host
-    sampler (kgvae/utils.py:79-124,158-171), not numpy's random stream."""
+    sampler (kgvae/utils.py:79-124,158-171), not numpy's random stream.
 
-    def __init__(self, triplets, sample_size, split_size, num_rels, negative_rate):
+    ``edge_sampler="neighbor"``: the B picks are the next row of a ``NeighborEdgeBank`` (the reference's
+    neighbourhood-expansion sampler) instead; everything downstream is the same.  Call ``before_replay()`` before each
+    replay of a captured ``sample()`` (``CapturedTrainStep.step`` does)."""
+
+    def __init__(self, triplets, sample_size, split_size, num_rels, negative_rate, edge_sampler="uniform"):
         if not triplets.is_cuda:
             raise RuntimeError("SampledDeviceSampler needs the triples on a CUDA device (no CPU fallback)")
         self.triplets = triplets.to(torch.int32).contiguous()
@@ -272,11 +334,22 @@ class SampledDeviceSampler:
         self.labels = torch.zeros(self.B * (self.rate + 1), dtype=torch.float32, device=dev)
         self.labels[:self.B] = 1
         self.n_edges, self.n_samples = 2 * self.keep_n, self.B * (self.rate + 1)
+        if edge_sampler not in ("uniform", "neighbor"):
+            raise ValueError("Sampler type must be either 'uniform' or 'neighbor'.")
+        self.bank = NeighborEdgeBank(self.triplets, self.num_nodes, self.B) if edge_sampler == "neighbor" else None
+
+    def before_replay(self):
+        if self.bank is not None:
+            self.bank.before_replay()
 
     def sample(self):
         dev = self.triplets.device
-        picked = torch.argsort(torch.rand(self.triplets.shape[0], device=dev))[:self.B]
-        node_id, src, rel, dst, n_valid = ops.sample_relabel(self.triplets[picked], self.num_nodes, self.n)
+        if self.bank is not None:
+            picked = self.bank.next()
+        else:
+            picked = torch.argsort(torch.rand(self.triplets.shape[0], device=dev))[:self.B]
+        node_id, src, rel, dst, n_valid = ops.sample_relabel(self.triplets.index_select(0, picked), self.num_nodes,
+                                                              self.n)
         pos = torch.stack([src, rel, dst], dim=1)
         m = self.B * self.rate
         # floor(u n_valid) with u in [0, 1) drawn in double: below n_valid for any n_valid < 2^24

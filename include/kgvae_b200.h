@@ -79,6 +79,27 @@ int kg_sample_relabel(const int32_t* picked, int n_picks, int num_nodes, int cap
                       int32_t* src, int32_t* rel, int32_t* dst, int32_t* n_valid,
                       void* workspace, size_t workspace_bytes, void* stream);
 
+/* Neighbourhood-expansion edge sampler (new device form of utils.sample_edge_neighborhood, kgvae/utils.py:33-76):
+ * one launch draws n_samples independent samples of sample_size distinct triples, one warp per sample.  Each pick
+ * consumes KG_NEIGHBOR_WORDS caller words: word 0 draws the vertex (~ cnt * seen, or ~ [cnt > 0] when that sums to
+ * 0), words 1..KG_NEIGHBOR_TRIES are the reference's rejection tries on its adjacency list, the next word picks
+ * among its unpicked entries when every try hit a picked edge.  tests/neighbor_mirror.py is the specification; the
+ * output depends only on the graph and the words.
+ *   adj_ptr [N+1], adj [2T][2] (edge id, other end): per entity, ascending edge id, the subject end first for a
+ *                  self-loop (utils.get_adj_and_degrees)
+ *   words [n_samples, sample_size, KG_NEIGHBOR_WORDS] uniform 32-bit, picks [n_samples, sample_size] edge ids,
+ *   fallbacks [n_samples] (or NULL): picks that needed the unpicked-entry scan
+ * The per-sample state lives in shared memory when it fits, else in the workspace (one slab per resident warp).
+ * kg_neighbor_sample_plan gives the samples resident in one wave (bounded by a 1 GiB budget for words, picks and
+ * slabs) and the workspace bytes for that many.  Needs 1 <= sample_size <= T and 0 < N, T < 2^30. */
+#define KG_NEIGHBOR_WORDS 8
+#define KG_NEIGHBOR_TRIES 6
+int kg_neighbor_sample_plan(int num_nodes, int n_triples, int sample_size, int* samples_per_launch,
+                            size_t* workspace_bytes);
+int kg_neighbor_sample(const int32_t* adj_ptr, const int32_t* adj, int num_nodes, int n_triples, int sample_size,
+                       int n_samples, const uint32_t* words, int32_t* picks, int32_t* fallbacks,
+                       void* workspace, size_t workspace_bytes, void* stream);
+
 /* Same index structures from an edge list the caller already ordered (the DGLGraph
  * surface: g.add_edges(src, dst) + etypes + per-edge norm, kgvae/utils.py:141-148).
  * Edges need not be sorted; the original edge order is kept as the tie-break so the

@@ -12,6 +12,7 @@ import torch
 import torch.nn as nn
 
 from . import datasets, ops, utils
+from .graph import Graph
 from .model import KGVAE, RGCN
 
 
@@ -143,6 +144,24 @@ class LinkPredict(nn.Module):
         return loss, predict_loss, kl, mmd
 
 
+def _step_forward(model, buckets, g, node_id, etype, norm, samples, labels):
+    """First half of the train step of kgvae/link_predict.py:217-228: zero the gradient buckets, forward, ``get_loss``.
+    Returns (loss, predict_loss, kl, mmd)."""
+    buckets.zero()
+    embed = model(g, node_id, etype, norm)
+    return model.get_loss(g, embed, samples, labels)
+
+
+def _step_update(model, buckets, optimizer, loss, grad_norm):
+    """Second half: backward, clipping, Adam.  Then the tensors the encoder caches drop the step's autograd graph,
+    which a capture on another stream needs (LinkPredict.release_graph)."""
+    loss.backward()
+    buckets.finish()
+    buckets.clip_(grad_norm)
+    optimizer.step()
+    model.release_graph()
+
+
 class CapturedTrainStep:
     """The train step of kgvae/link_predict.py:217-228 - edge index, forward, ``get_loss``, backward,
     ``clip_grad_norm_``, ``optimizer.step()`` - for inputs of FIXED shape (full-graph training, or any fixed
@@ -174,13 +193,11 @@ class CapturedTrainStep:
 
     def __init__(self, model, optimizer, example, num_nodes, buckets=None, grad_norm=1.0, warmup=3, sampler=None):
         from . import _lib
-        from .graph import Graph
         if not all(g.get("capturable", False) for g in optimizer.param_groups):
             raise RuntimeError("CapturedTrainStep: the optimizer must be constructed with capturable=True")
         dev = example["src"].device if example is not None else next(model.parameters()).device
         if dev.type != "cuda":
             raise RuntimeError("kgvae_b200: CapturedTrainStep needs CUDA tensors (no CPU fallback)")
-        self._Graph = Graph
         self.model, self.optimizer, self.num_nodes, self.grad_norm = model, optimizer, int(num_nodes), grad_norm
         self.buckets = buckets if buckets is not None else model.grad_buckets()
         self.sampler = sampler
@@ -210,16 +227,11 @@ class CapturedTrainStep:
 
     def _eager(self):
         t = self.inputs if self.sampler is None else self.sampler.sample()
-        g = self._Graph.from_device_edges(self.num_nodes, t["src"], t["dst"])
+        g = Graph.from_device_edges(self.num_nodes, t["src"], t["dst"])
         g.n_valid = t.get("n_valid")
-        self.buckets.zero()
-        embed = self.model(g, t["node_id"], t["etype"], t["norm"])
-        loss, self.predict_loss, self.kl, self.mmd = self.model.get_loss(g, embed, t["samples"], t["labels"])
-        loss.backward()
-        self.buckets.finish()
-        self.buckets.clip_(self.grad_norm)
-        self.optimizer.step()
-        self.model.release_graph()
+        loss, self.predict_loss, self.kl, self.mmd = _step_forward(self.model, self.buckets, g, t["node_id"],
+                                                                   t["etype"], t["norm"], t["samples"], t["labels"])
+        _step_update(self.model, self.buckets, self.optimizer, loss, self.grad_norm)
         return loss.detach()
 
     def close(self):
@@ -282,6 +294,44 @@ def _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val
     return best_mrr
 
 
+def _batch_sampler(args, train_data, num_nodes, num_rels, device):
+    """The sampler of the eager loop (kgvae/utils.py:79-124): a callable that draws the next training batch as
+    ``(g, node_id, edge_type, edge_norm, samples, labels)`` on ``device``.  By default the host sampler on numpy's
+    global stream; with --device-sampler the same procedure drawn on the GPU (not numpy's random stream)."""
+    if getattr(args, "device_sampler", False):
+        train_dev = torch.from_numpy(np.asarray(train_data)).to(device)
+        bank = None                      # its constructor draws nothing: the first draw refills it
+        if args.edge_sampler == "neighbor" and args.graph_batch_size < len(train_data):
+            bank = utils.NeighborEdgeBank(train_dev, num_nodes, args.graph_batch_size)
+        return lambda: utils.generate_sampled_graph_and_labels_device(
+            train_dev, args.graph_batch_size, args.graph_split_size, num_rels, args.negative_sample,
+            picked=None if bank is None else bank.next())
+    adj_list, degrees = utils.get_adj_and_degrees(num_nodes, train_data)
+
+    def draw():
+        g, node_id, edge_type, node_norm, samples, labels = utils.generate_sampled_graph_and_labels(
+            train_data, args.graph_batch_size, args.graph_split_size, num_rels, adj_list, degrees,
+            args.negative_sample, args.edge_sampler)
+        node_id = torch.from_numpy(node_id).view(-1, 1).long().to(device)
+        edge_type = torch.from_numpy(edge_type).to(device)
+        edge_norm = node_norm_to_edge_norm(g, torch.from_numpy(node_norm).view(-1, 1)).to(device)
+        samples, labels = torch.from_numpy(samples).to(device), torch.from_numpy(labels).to(device)
+        return g, node_id, edge_type, edge_norm, samples, labels
+    return draw
+
+
+def _capturable_sampler(args, train_data, num_rels, device):
+    """The sampler --capture-step captures with the step: its draws have fixed shapes, so sampler + step are captured
+    once and every iteration is one CUDA-graph replay.  Full-graph training scores all training triples with fresh
+    negatives on a fresh graph split (both edge samplers select every triple when B >= T); sampled subgraphs
+    (--device-sampler) pad the node set to a fixed budget."""
+    train_dev = torch.from_numpy(np.asarray(train_data)).to(device)
+    if args.graph_batch_size >= len(train_data):
+        return utils.FullBatchDeviceSampler(train_dev, num_rels, args.negative_sample, args.graph_split_size)
+    return utils.SampledDeviceSampler(train_dev, args.graph_batch_size, args.graph_split_size, num_rels,
+                                      args.negative_sample, edge_sampler=args.edge_sampler)
+
+
 def main(args):
     data = datasets.load_data(args.dataset)
     num_nodes, num_rels = data.num_nodes, data.num_rels
@@ -301,7 +351,6 @@ def main(args):
     valid_t = torch.LongTensor(valid_data)
     val_graph, val_rel, val_norm = utils.build_test_graph(num_nodes, num_rels, valid_t)
     val_node_id, val_rel, val_norm = _graph_inputs(val_graph, val_rel, val_norm, num_nodes, device)
-    adj_list, degrees = utils.get_adj_and_degrees(num_nodes, train_data)
     capture = bool(getattr(args, "capture_step", False))
     optimizer = torch.optim.Adam(model.parameters(), lr=args.lr, fused=True, capturable=capture)
     # gradients live in one flat buffer: zeroing is one memset, clipping one norm + one scale
@@ -337,87 +386,47 @@ def main(args):
         model.load_state_dict(checkpoint["state_dict"])
         epoch = checkpoint["epoch"]
 
-    train_dev = None
-    captured = None
-    bank = None                          # eager --device-sampler --edge-sampler neighbor: a bank of edge samples
+    if args.edge_sampler not in ("uniform", "neighbor"):
+        raise ValueError("Sampler type must be either 'uniform' or 'neighbor'.")
+    if capture and not (args.graph_batch_size >= len(train_data) or getattr(args, "device_sampler", False)):
+        raise RuntimeError("--capture-step needs full-batch sampling (--graph-batch-size >= the number of "
+                           f"training triples, {len(train_data)}) or --device-sampler")
+    model.train()
     if capture:
-        # full-graph training: every iteration scores all training triples with fresh negatives on a fresh graph
-        # split - fixed shapes, so sampler + step are captured once and every iteration is one CUDA-graph replay.
-        # Sampled subgraphs (--device-sampler): the node set is padded to a fixed budget, so their shapes are fixed too
-        # Both edge samplers select every triple when B >= T, so FullBatchDeviceSampler serves both there
-        full = args.graph_batch_size >= len(train_data)
-        sampled = getattr(args, "device_sampler", False)
-        if args.edge_sampler not in ("uniform", "neighbor"):
-            raise ValueError("Sampler type must be either 'uniform' or 'neighbor'.")
-        if not (full or sampled):
-            raise RuntimeError("--capture-step needs full-batch sampling (--graph-batch-size >= the number of "
-                               f"training triples, {len(train_data)}) or --device-sampler")
-        model.train()
-        train_dev = torch.from_numpy(np.asarray(train_data)).to(device)
-        if full:
-            sampler = utils.FullBatchDeviceSampler(train_dev, num_rels, args.negative_sample, args.graph_split_size)
-        else:
-            sampler = utils.SampledDeviceSampler(train_dev, args.graph_batch_size, args.graph_split_size, num_rels,
-                                                 args.negative_sample, edge_sampler=args.edge_sampler)
+        sampler = _capturable_sampler(args, train_data, num_rels, device)
         captured = CapturedTrainStep(model, optimizer, None, sampler.n, buckets=buckets, grad_norm=args.grad_norm,
                                      warmup=1, sampler=sampler)
         epoch += 1                       # the warm-up step that precedes the capture is a training step
-    while True:
-        model.train()
-        epoch += 1
-        if captured is not None:
+
+        def train_step():
             torch.cuda.synchronize()
             t0 = time.time()
             loss = captured.step()
             torch.cuda.synchronize()
-            forward_time.append(time.time() - t0)          # the replay is forward + backward + update in one
-            backward_time.append(0.0)
-            print("Epoch {:04d} | Loss {:.4f} | Best MRR {:.4f} | pred_loss {:.4f} | kl {:.4f} | mmd {:.4f}".format(
-                epoch, loss.item(), best_mrr, captured.predict_loss.item(), captured.kl.item(), captured.mmd.item()))
-            if epoch % args.evaluate_every == 0:
-                best_mrr = _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t)
-            if epoch >= args.n_epochs:
-                break
-            continue
-        if getattr(args, "device_sampler", False) and args.edge_sampler in ("uniform", "neighbor"):
-            # opt-in: the same sampling procedure drawn on the GPU (not numpy's random stream)
-            if train_dev is None:
-                train_dev = torch.from_numpy(np.asarray(train_data)).to(device)
-            picked = None
-            if args.edge_sampler == "neighbor" and args.graph_batch_size < len(train_data):
-                if bank is None:
-                    bank = utils.NeighborEdgeBank(train_dev, num_nodes, args.graph_batch_size)
-                picked = bank.next()
-            g, node_id, edge_type, edge_norm, batch, labels = utils.generate_sampled_graph_and_labels_device(
-                train_dev, args.graph_batch_size, args.graph_split_size, num_rels, args.negative_sample,
-                picked=picked)
-        else:
-            g, node_id, edge_type, node_norm, batch, labels = utils.generate_sampled_graph_and_labels(
-                train_data, args.graph_batch_size, args.graph_split_size, num_rels, adj_list, degrees,
-                args.negative_sample, args.edge_sampler)
-            node_id = torch.from_numpy(node_id).view(-1, 1).long().to(device)
-            edge_type = torch.from_numpy(edge_type).to(device)
-            edge_norm = node_norm_to_edge_norm(g, torch.from_numpy(node_norm).view(-1, 1)).to(device)
-            batch, labels = torch.from_numpy(batch).to(device), torch.from_numpy(labels).to(device)
+            # the replay is forward + backward + update in one: all of it counts as forward time
+            return (loss, captured.predict_loss, captured.kl, captured.mmd), time.time() - t0, 0.0
+    else:
+        draw = _batch_sampler(args, train_data, num_nodes, num_rels, device)
 
-        torch.cuda.synchronize()
-        t0 = time.time()
-        embed = model(g, node_id, edge_type, edge_norm)
-        loss, pred_loss, kl, mmd = model.get_loss(g, embed, batch, labels)
-        torch.cuda.synchronize()
-        t1 = time.time()
-        loss.backward()
-        buckets.finish()
-        buckets.clip_(args.grad_norm)
-        optimizer.step()
-        torch.cuda.synchronize()
-        t2 = time.time()
-        forward_time.append(t1 - t0)
-        backward_time.append(t2 - t1)
+        def train_step():
+            g, node_id, edge_type, edge_norm, samples, labels = draw()
+            torch.cuda.synchronize()
+            t0 = time.time()
+            terms = _step_forward(model, buckets, g, node_id, edge_type, edge_norm, samples, labels)
+            torch.cuda.synchronize()
+            t1 = time.time()
+            _step_update(model, buckets, optimizer, terms[0], args.grad_norm)
+            torch.cuda.synchronize()
+            return terms, t1 - t0, time.time() - t1
+
+    while True:
+        model.train()
+        epoch += 1
+        (loss, pred_loss, kl, mmd), t_forward, t_backward = train_step()
+        forward_time.append(t_forward)
+        backward_time.append(t_backward)
         print("Epoch {:04d} | Loss {:.4f} | Best MRR {:.4f} | pred_loss {:.4f} | kl {:.4f} | mmd {:.4f}".format(
             epoch, loss.item(), best_mrr, pred_loss.item(), kl.item(), mmd.item()))
-        buckets.zero()
-
         if epoch % args.evaluate_every == 0:
             best_mrr = _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t)
         if epoch >= args.n_epochs:

@@ -24,7 +24,7 @@ int kg_fail(int code, const char* fmt, ...) {
 }
 
 extern "C" const char* kg_last_error(void) { return g_err; }
-extern "C" int kg_version(void) { return 100; }
+extern "C" int kg_version(void) { return 101; }
 
 int kg_sm_count() {
   static int cached[64] = {0};            // per device: a process may drive several GPUs
@@ -41,9 +41,9 @@ int kg_sm_count() {
 
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is per device: remember which devices have it for `slot`
 bool kg_attr_needed(int slot) {
-  static unsigned long long done[8] = {0};
+  static unsigned long long done[16] = {0};
   int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64 || slot < 0 || slot >= 8) return true;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64 || slot < 0 || slot >= 16) return true;
   const unsigned long long bit = 1ull << dev;
   if (done[slot] & bit) return false;
   done[slot] |= bit;

@@ -276,6 +276,10 @@ filter_correction(const float* __restrict__ q32, const float* __restrict__ emb, 
 // fp32 dot product and keeps the k best by (score desc, entity id asc); a tile whose (k+1)-th listed score
 // could still reach the k-th exact score (within the filter's error band) is re-scanned completely, so
 // the result does not depend on the tensor-core rounding.
+// Filtered generation (FILT, an extension): each query's listed entities (ascending CSR) are scored -inf in the
+// tile epilogue, so every tile's list holds its best UNLISTED candidates and the error-band argument above holds
+// for the unlisted entities; the re-scan of a tile skips the listed ones too.  FILT = false is the unfiltered
+// kernel unchanged (the filter fields sit behind the ones it reads).
 // ------------------------------------------------------------------------------------------
 struct TopkArgs {
   const float2* colp;
@@ -283,7 +287,19 @@ struct TopkArgs {
   float* cand_v;
   int* cand_i;
   int M, Kp, n_cand, m_tiles, n_tiles, n_terms;
+  const int* filt_ptr;   // FILT only
+  const int* filt_idx;
 };
+
+// first position in v[lo, hi) whose value is >= key
+__device__ __forceinline__ int lower_bound_i32(const int* __restrict__ v, int lo, int hi, int key) {
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(v + mid) < key) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo;
+}
 
 template <int KK>
 __device__ __forceinline__ void topk_insert(float (&bv)[KK], int (&bi)[KK], float v, int n) {
@@ -299,7 +315,7 @@ __device__ __forceinline__ void topk_insert(float (&bv)[KK], int (&bi)[KK], floa
   }
 }
 
-template <int KK>
+template <int KK, bool FILT>
 __global__ void __launch_bounds__(THREADS, 1)
 topk_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, TopkArgs p) {
   extern __shared__ uint8_t smem_raw[];
@@ -329,16 +345,34 @@ topk_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
 #pragma unroll
       for (int i = 0; i < KK; ++i) { bv[i] = -INFINITY; bi[i] = -1; }
       const float2* cs = colp_s + buf * BN;
+      int fc = 0, fe = 0;            // FILT: cursor into this row's list, at its first id >= n0
+      if constexpr (FILT) {
+        if (m < p.M) {
+          fe = __ldg(p.filt_ptr + m + 1);
+          fc = lower_bound_i32(p.filt_idx, __ldg(p.filt_ptr + m), fe, n0);
+        }
+      }
 #pragma unroll 1
       for (int c = 0; c < BN / 32; ++c) {
         uint32_t v[32];
         tmem_ld_32x32b_x32(taddr + c * 32, v);
+        uint32_t listed = 0;           // FILT: bit j = entity n0 + 32 c + j is listed
+        if constexpr (FILT) {
+          for (; fc < fe; ++fc) {
+            const int j = __ldg(p.filt_idx + fc) - (n0 + c * 32);
+            if (j >= 32) break;
+            if (j >= 0) listed |= 1u << j;
+          }
+        }
         tmem_ld_wait();
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           const float2 cp = cs[c * 32 + j];                                    // {1 / s_e, |e|}: broadcast
           const int n = n0 + c * 32 + j;
-          const float val = n < p.n_cand ? __uint_as_float(v[j]) * cp.x * inv_sq : -INFINITY;
+          float val = n < p.n_cand ? __uint_as_float(v[j]) * cp.x * inv_sq : -INFINITY;
+          if constexpr (FILT) {
+            if ((listed >> j) & 1u) val = -INFINITY;
+          }
           topk_insert<KK>(bv, bi, val, n);
         }
       }
@@ -371,12 +405,15 @@ colp_max_kernel(const float2* __restrict__ colp, int n_cand, float* __restrict__
 
 constexpr int kTopkMax = 10;
 
-// one warp per query; every lane keeps the same sorted list (scores are warp-uniform after the butterfly sum)
+// one warp per query; every lane keeps the same sorted list (scores are warp-uniform after the butterfly sum).
+// FILT: the tiles' candidate lists hold no listed entity (the epilogue scored them -inf), the re-scan skips them.
+template <bool FILT>
 __global__ void __launch_bounds__(256)
 topk_finish_kernel(const float* __restrict__ q32, const float* __restrict__ emb, const float4* __restrict__ rowp,
                    const float* __restrict__ sqv, const float* __restrict__ cand_v, const int* __restrict__ cand_i,
                    const float* __restrict__ emax_p, int M, int h, int n_cand, int n_tiles, int KK, int k,
-                   const float* __restrict__ shift_p, int* __restrict__ out_idx, float* __restrict__ out_score) {
+                   const float* __restrict__ shift_p, int* __restrict__ out_idx, float* __restrict__ out_score,
+                   const int* __restrict__ filt_ptr, const int* __restrict__ filt_idx) {
   const int m = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (m >= M) return;
   const float shift = shift_p ? __ldg(shift_p) : 0.f;
@@ -416,7 +453,24 @@ topk_finish_kernel(const float* __restrict__ q32, const float* __restrict__ emb,
     const float v_last = __ldg(cv + t * KK + KK - 1);        // the best score NOT kept is <= this one
     if (!(v_last + shift + band >= ts[k - 1])) continue;
     const int n_end = min(n_cand, (t + 1) * BN);
-    for (int n = t * BN; n < n_end; ++n) offer(warp_dot(q, emb + (size_t)n * h, h, lane) + shift, n);
+    int fc = 0, fe = 0, nx = 0x7fffffff;        // FILT: the row's next listed id >= n (warp-uniform)
+    if constexpr (FILT) {
+      fe = __ldg(filt_ptr + m + 1);
+      fc = lower_bound_i32(filt_idx, __ldg(filt_ptr + m), fe, t * BN);
+      nx = fc < fe ? __ldg(filt_idx + fc) : 0x7fffffff;
+    }
+    for (int n = t * BN; n < n_end; ++n) {
+      if constexpr (FILT) {
+        bool listed = false;
+        while (nx <= n) {
+          listed |= nx == n;
+          ++fc;
+          nx = fc < fe ? __ldg(filt_idx + fc) : 0x7fffffff;
+        }
+        if (listed) continue;
+      }
+      offer(warp_dot(q, emb + (size_t)n * h, h, lane) + shift, n);
+    }
   }
   if (lane == 0)
     for (int i = 0; i < k; ++i) {
@@ -524,11 +578,12 @@ extern "C" size_t kg_distmult_topk_workspace_bytes(int n_queries, int n_entities
 }
 
 // out_idx [n_queries, k] int32 (entity ids, best first; -1 when fewer than k entities), out_score [n_queries, k]
-// fp32 canonical scores (+ shift): the k highest-scored tails of each query (a_i, r_i) among ALL entities.
-extern "C" int kg_distmult_topk(const float* emb, const float* w, const int32_t* a, const int32_t* r,
-                                int n_queries, int n_entities, int h, const float* shift, int k,
-                                void* workspace, size_t workspace_bytes, int32_t* out_idx, float* out_score,
-                                void* stream) {
+// fp32 canonical scores (+ shift): the k highest-scored tails of each query (a_i, r_i) among ALL entities, or among
+// the entities not in the query's filter list (filt_ptr != nullptr).
+static int topk_impl(const float* emb, const float* w, const int32_t* a, const int32_t* r, int n_queries,
+                     int n_entities, int h, const float* shift, int k, const int32_t* filt_ptr,
+                     const int32_t* filt_idx, void* workspace, size_t workspace_bytes, int32_t* out_idx,
+                     float* out_score, void* stream) {
   KG_REQUIRE(n_queries >= 0 && n_entities > 0 && h > 0, "topk: bad sizes");
   KG_REQUIRE(k >= 1 && k <= kTopkMax, "topk: k must be in 1..10");
   cudaStream_t st = kg_stream(stream);
@@ -572,21 +627,50 @@ extern "C" int kg_distmult_topk(const float* emb, const float* w, const int32_t*
   args.colp = colp; args.sqv = sqv; args.cand_v = cand_v; args.cand_i = cand_i;
   args.M = M; args.Kp = L.Kp; args.n_cand = n_cand; args.m_tiles = L.m_tiles; args.n_tiles = L.n_tiles;
   args.n_terms = n_terms;
+  args.filt_ptr = filt_ptr; args.filt_idx = filt_idx;
   const int total = L.m_tiles * L.n_tiles;
   const int grid = total < kg_sm_count() ? total : kg_sm_count();
-#define KG_TOPK_LAUNCH(KK_, SLOT_)                                                                              \
+#define KG_TOPK_LAUNCH(KK_, FILT_, SLOT_)                                                                       \
   do {                                                                                                          \
     if (kg_attr_needed(SLOT_))                                                                                  \
-      KG_CUDA(cudaFuncSetAttribute(topk_tc_kernel<KK_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)); \
-    topk_tc_kernel<KK_><<<grid, THREADS, SMEM_BYTES, st>>>(tm_a, tm_b, args);                                   \
+      KG_CUDA(cudaFuncSetAttribute(topk_tc_kernel<KK_, FILT_>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
+                                   SMEM_BYTES));                                                                \
+    topk_tc_kernel<KK_, FILT_><<<grid, THREADS, SMEM_BYTES, st>>>(tm_a, tm_b, args);                            \
   } while (0)
-  if (KK == 2) KG_TOPK_LAUNCH(2, 2);
-  else if (KK == 4) KG_TOPK_LAUNCH(4, 3);
-  else KG_TOPK_LAUNCH(kTopkMax + 1, 4);
+  const int fgrid = kg_div_up((long long)M * 32, 256);
+  if (filt_ptr == nullptr) {
+    if (KK == 2) KG_TOPK_LAUNCH(2, false, 2);
+    else if (KK == 4) KG_TOPK_LAUNCH(4, false, 3);
+    else KG_TOPK_LAUNCH(kTopkMax + 1, false, 4);
+    KG_LAUNCH_OK();
+    topk_finish_kernel<false><<<fgrid, 256, 0, st>>>(q32, emb, rowp, sqv, cand_v, cand_i, emax, M, h, n_cand,
+                                                     L.n_tiles, KK, k, shift, out_idx, out_score, nullptr, nullptr);
+  } else {
+    if (KK == 2) KG_TOPK_LAUNCH(2, true, 6);
+    else if (KK == 4) KG_TOPK_LAUNCH(4, true, 7);
+    else KG_TOPK_LAUNCH(kTopkMax + 1, true, 8);
+    KG_LAUNCH_OK();
+    topk_finish_kernel<true><<<fgrid, 256, 0, st>>>(q32, emb, rowp, sqv, cand_v, cand_i, emax, M, h, n_cand,
+                                                    L.n_tiles, KK, k, shift, out_idx, out_score, filt_ptr, filt_idx);
+  }
 #undef KG_TOPK_LAUNCH
   KG_LAUNCH_OK();
-  topk_finish_kernel<<<kg_div_up((long long)M * 32, 256), 256, 0, st>>>(
-      q32, emb, rowp, sqv, cand_v, cand_i, emax, M, h, n_cand, L.n_tiles, KK, k, shift, out_idx, out_score);
-  KG_LAUNCH_OK();
   return KG_OK;
+}
+
+extern "C" int kg_distmult_topk(const float* emb, const float* w, const int32_t* a, const int32_t* r,
+                                int n_queries, int n_entities, int h, const float* shift, int k,
+                                void* workspace, size_t workspace_bytes, int32_t* out_idx, float* out_score,
+                                void* stream) {
+  return topk_impl(emb, w, a, r, n_queries, n_entities, h, shift, k, nullptr, nullptr, workspace, workspace_bytes,
+                   out_idx, out_score, stream);
+}
+
+extern "C" int kg_distmult_topk_filtered(const float* emb, const float* w, const int32_t* a, const int32_t* r,
+                                         int n_queries, int n_entities, int h, const float* shift, int k,
+                                         const int32_t* filt_ptr, const int32_t* filt_idx, void* workspace,
+                                         size_t workspace_bytes, int32_t* out_idx, float* out_score, void* stream) {
+  KG_REQUIRE(filt_ptr != nullptr && filt_idx != nullptr, "topk filtered: needs both filt_ptr and filt_idx");
+  return topk_impl(emb, w, a, r, n_queries, n_entities, h, shift, k, filt_ptr, filt_idx, workspace, workspace_bytes,
+                   out_idx, out_score, stream);
 }

@@ -275,8 +275,10 @@ def _graph_inputs(graph, rel, norm, num_nodes, device):
     return node_id, rel_t, edge_norm
 
 
-def _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t):
-    """Periodic validation with checkpoints (kgvae/link_predict.py:238-259); returns the best MRR so far."""
+def _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t, filter_index=None):
+    """Periodic validation with checkpoints (kgvae/link_predict.py:238-259); returns the best MRR so far.  With
+    ``filter_index`` the filtered metrics of the same embedding are printed too; the checkpoint choice stays on the
+    raw MRR, as in the reference."""
     model.eval()
     print("start eval")
     torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file)
@@ -285,6 +287,9 @@ def _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val
     mrr = utils.calc_mrr(embed, model.w_relation, valid_t, hits=[1, 3, 10],
                          eval_bz=args.eval_batch_size, all_batches=False,
                          flow_log_prob=model._flow_shift())
+    if filter_index is not None:
+        utils.calc_mrr(embed, model.w_relation, valid_t, hits=[1, 3, 10], eval_bz=args.eval_batch_size,
+                       all_batches=False, flow_log_prob=model._flow_shift(), filter_index=filter_index)
     model.release_graph()
     if mrr < best_mrr:
         torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file + "_latest")
@@ -349,6 +354,10 @@ def main(args):
                         n_flows=args.n_flows).to(device)
 
     valid_t = torch.LongTensor(valid_data)
+    filter_index = None
+    if getattr(args, "filtered", False):       # every known triple: train + valid + test
+        filter_index = utils.FilterIndex(np.concatenate([train_data, valid_data, test_data]), num_nodes, num_rels,
+                                         device)
     val_graph, val_rel, val_norm = utils.build_test_graph(num_nodes, num_rels, valid_t)
     val_node_id, val_rel, val_norm = _graph_inputs(val_graph, val_rel, val_norm, num_nodes, device)
     capture = bool(getattr(args, "capture_step", False))
@@ -371,12 +380,16 @@ def main(args):
             embed = model(test_graph, test_node_id, test_rel, test_norm)
         if args.generate:             # kgvae/link_predict.py:181-184: generation instead of ranking
             tails, scores = utils.generate(embed, model.w_relation, test_t, flow_log_prob=model._flow_shift(),
-                                           out_path="result.txt")
+                                           out_path="result.txt", filter_index=filter_index)
             print(f"generated tails for {len(tails)} test queries -> result.txt")
             return tails
-        return utils.calc_mrr(embed, model.w_relation, test_t, hits=[1, 3, 10],
-                              eval_bz=args.eval_batch_size, all_batches=True,
-                              flow_log_prob=model._flow_shift())
+        mrr = utils.calc_mrr(embed, model.w_relation, test_t, hits=[1, 3, 10],
+                             eval_bz=args.eval_batch_size, all_batches=True,
+                             flow_log_prob=model._flow_shift())
+        if filter_index is not None:
+            utils.calc_mrr(embed, model.w_relation, test_t, hits=[1, 3, 10], eval_bz=args.eval_batch_size,
+                           all_batches=True, flow_log_prob=model._flow_shift(), filter_index=filter_index)
+        return mrr
 
     print("start training...")
     epoch, best_mrr = 0, 0
@@ -428,7 +441,8 @@ def main(args):
         print("Epoch {:04d} | Loss {:.4f} | Best MRR {:.4f} | pred_loss {:.4f} | kl {:.4f} | mmd {:.4f}".format(
             epoch, loss.item(), best_mrr, pred_loss.item(), kl.item(), mmd.item()))
         if epoch % args.evaluate_every == 0:
-            best_mrr = _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t)
+            best_mrr = _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t,
+                                 filter_index)
         if epoch >= args.n_epochs:
             break
 
@@ -474,6 +488,11 @@ def build_parser():
                    help="(new) draw the edge sample (--edge-sampler uniform or neighbor), the negatives and the "
                         "graph split on the GPU; same procedure as the reference's host sampler, not its numpy random "
                         "stream.  The neighbour sampler draws a bank of samples per kernel launch")
+    p.add_argument("--filtered", action="store_true",
+                   help="(new) also report filtered MRR / Hits@k - every other entity that forms a train, valid or "
+                        "test triple with a query is left out of its rank - after the raw ones (--test-mode and "
+                        "periodic validation; checkpoints are still chosen on the raw MRR), and make --generate "
+                        "write only tails that form no known triple.  The filter lists are built on the GPU once")
     return p
 
 

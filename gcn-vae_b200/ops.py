@@ -1001,10 +1001,14 @@ def distmult_rank(emb, w, a, r, b, shift=None, cand_range=None, filt_ptr=None, f
     return ranks[:M]
 
 
-def distmult_topk(emb, w, a, r, k=1, shift=None):
+def distmult_topk(emb, w, a, r, k=1, shift=None, filt_ptr=None, filt_idx=None):
     """The ``k`` highest-scored tails of each query (a_i, r_i) among all entities, best first (ties by ascending
     entity id): utils.generate's ``score.argmax`` (kgvae/utils.py:245-288) generalised to top-k, without the
-    score matrix.  Returns (idx int32 [M, k], score fp32 [M, k])."""
+    score matrix.  ``filt_ptr`` / ``filt_idx``: per-query CSR of entities to leave out (ascending, duplicate-free;
+    ``filter_lists``); a query with fewer than k other entities gets trailing -1.
+    Returns (idx int32 [M, k], score fp32 [M, k])."""
+    if (filt_ptr is None) != (filt_idx is None):
+        raise ValueError("distmult_topk: a filter needs both filt_ptr and filt_idx")
     emb, w = _c(emb.detach()), _c(w.detach())
     M, (V, h) = a.numel(), emb.shape
     dev = emb.device
@@ -1012,6 +1016,47 @@ def distmult_topk(emb, w, a, r, k=1, shift=None):
     score = torch.empty((max(M, 1), k), dtype=torch.float32, device=dev)
     ws = L.workspace(L.lib().kg_distmult_topk_workspace_bytes(M, V, h, k), dev)
     sh = None if shift is None else _c(torch.as_tensor(shift, dtype=torch.float32, device=dev).reshape(1))
-    L.call("kg_distmult_topk", L.f32(emb), L.f32(w), L.i32(a), L.i32(r), M, V, h, L.f32(sh), int(k),
-           L.ptr(ws), ws.numel(), L.i32(idx), L.f32(score), L.stream())
+    head = (L.f32(emb), L.f32(w), L.i32(a), L.i32(r), M, V, h, L.f32(sh), int(k))
+    tail = (L.ptr(ws), ws.numel(), L.i32(idx), L.f32(score), L.stream())
+    if filt_ptr is None:
+        L.call("kg_distmult_topk", *head, *tail)
+    else:
+        L.call("kg_distmult_topk_filtered", *head, L.i32(filt_ptr), L.i32(filt_idx), *tail)
     return idx[:M], score[:M]
+
+
+# ---------------------------------------------------------------------------------------------
+# filter lists (device counterpart of utils.build_filter)
+# ---------------------------------------------------------------------------------------------
+FILTER_DIRECTIONS = {"object": 0, "subject": 1}     # KG_FILTER_OBJECT / KG_FILTER_SUBJECT of include/kgvae_b200.h
+
+
+def filter_table(triplets, num_nodes, num_rels, direction):
+    """kg_filter_table: the sorted, duplicate-free keys (a R + r) N + c of the known ``triplets`` (int tensor [T, 3]
+    (s, r, o) on the device), a = s and c = o for ``direction="object"``, the other way round for "subject".
+    Returns (table int64 [max(T, 1)], table_len int32 [1]) on the device."""
+    tri = as_i32(triplets)
+    dev, T = tri.device, int(tri.shape[0])
+    table = torch.empty(max(T, 1), dtype=torch.int64, device=dev)
+    n = torch.empty(1, dtype=torch.int32, device=dev)
+    ws = L.workspace(L.lib().kg_filter_table_workspace_bytes(T), dev)
+    L.call("kg_filter_table", L.i32(tri), T, int(num_nodes), int(num_rels), FILTER_DIRECTIONS[direction],
+           L.ptr(table, torch.int64), L.i32(n), L.ptr(ws), ws.numel(), L.stream())
+    return table, n
+
+
+def filter_lists(table, table_len, num_nodes, num_rels, a, r):
+    """kg_filter_count + kg_filter_gather: for queries (a_i, r_i) (int32 device tensors) the CSR (ptr int32 [M+1],
+    idx int32 [ptr[M]]) of the entities their runs of ``table`` list - what utils.build_filter returns.  Reads the
+    total back once to size idx."""
+    a, r = as_i32(a), as_i32(r)
+    dev, M = a.device, int(a.numel())
+    ptr = torch.empty(M + 1, dtype=torch.int32, device=dev)
+    total = ctypes.c_longlong()
+    ws = L.workspace(L.lib().kg_filter_count_workspace_bytes(M), dev)
+    L.call("kg_filter_count", L.ptr(table, torch.int64), L.i32(table_len), int(num_nodes), int(num_rels),
+           L.i32(a), L.i32(r), M, L.i32(ptr), ctypes.byref(total), L.ptr(ws), ws.numel(), L.stream())
+    idx = torch.empty(max(total.value, 1), dtype=torch.int32, device=dev)
+    L.call("kg_filter_gather", L.ptr(table, torch.int64), L.i32(table_len), int(num_nodes), int(num_rels),
+           L.i32(a), L.i32(r), M, L.i32(ptr), L.i32(idx), L.stream())
+    return ptr, idx[:total.value]

@@ -393,24 +393,34 @@ def perturb_and_get_rank(embedding, w, a, r, b, test_size, batch_size=100, all_b
 
 
 def calc_mrr(embedding, w, test_triplets, hits=[], eval_bz=100, all_batches=True, flow_log_prob=None,
-             verbose=True, return_ranks=False):
-    """Raw MRR / Hits@k over both perturbation directions (utils.py:293-314)."""
+             verbose=True, return_ranks=False, filter_index=None):
+    """Raw MRR / Hits@k over both perturbation directions (utils.py:293-314).  With ``filter_index`` (a
+    ``FilterIndex``) the metrics are filtered instead (an extension; the reference is raw-only): every other
+    entity that forms a known triple with a query is left out of its rank."""
     with torch.no_grad():
         s, r, o = test_triplets[:, 0], test_triplets[:, 1], test_triplets[:, 2]
         n = test_triplets.shape[0]
-        ranks_s = perturb_and_get_rank(embedding, w, o, r, s, n, eval_bz, all_batches, flow_log_prob, verbose)
-        ranks_o = perturb_and_get_rank(embedding, w, s, r, o, n, eval_bz, all_batches, flow_log_prob, verbose)
+        filt_s = filt_o = None
+        if filter_index is not None:
+            m = n if all_batches else min(int(n), int(eval_bz))       # the queries perturb_and_get_rank ranks
+            filt_s = filter_index.lists(o[:m], r[:m], "subject")      # (c, r, o) known
+            filt_o = filter_index.lists(s[:m], r[:m], "object")       # (s, r, c) known
+        ranks_s = perturb_and_get_rank(embedding, w, o, r, s, n, eval_bz, all_batches, flow_log_prob, verbose,
+                                       filt=filt_s)
+        ranks_o = perturb_and_get_rank(embedding, w, s, r, o, n, eval_bz, all_batches, flow_log_prob, verbose,
+                                       filt=filt_o)
         ranks = torch.cat([ranks_s, ranks_o]) + 1
         mrr = torch.mean(1.0 / ranks.float())
         if verbose:
-            print("MRR (raw): {:.6f}".format(mrr.item()))
+            kind = "raw" if filter_index is None else "filtered"
+            print("MRR ({}): {:.6f}".format(kind, mrr.item()))
             for hit in hits:
-                print("Hits (raw) @ {}: {:.6f}".format(hit, torch.mean((ranks <= hit).float()).item()))
+                print("Hits ({}) @ {}: {:.6f}".format(kind, hit, torch.mean((ranks <= hit).float()).item()))
     return (mrr.item(), ranks) if return_ranks else mrr.item()
 
 
 def generate(embedding, w, test_triplets, eval_bz=200, topk=1, flow_log_prob=None, entity_names=None,
-             relation_names=None, out_path=None, max_lines=None):
+             relation_names=None, out_path=None, max_lines=None, filter_index=None):
     """Tail generation (kgvae/utils.py:245-288): for every test triple (a, r, b) the highest-scored tail(s) among
     all entities.  The reference scores 200 queries at a time through the D x E x V tensor, takes
     ``score.argmax`` and prints the triples around one hard-coded entity using name files from the author's home
@@ -418,13 +428,17 @@ def generate(embedding, w, test_triplets, eval_bz=200, topk=1, flow_log_prob=Non
     and ignored), and the triples are written as ids - or names, when ``entity_names`` / ``relation_names``
     (sequences or dicts indexed by id) are given - to ``out_path`` (default: nothing is written).
 
+    ``filter_index`` (a ``FilterIndex``; an extension): only tails c for which (a, r, c) is not a known triple are
+    returned - generation proposes new facts.  A query with fewer than ``topk`` such tails gets trailing -1.
+
     Returns (tails int64 [T, topk], scores fp32 [T, topk]) on the embedding's device; ``tails[:, 0]`` is the
     reference's ``highest_scored``."""
     with torch.no_grad():
         dev = embedding.device
         t = torch.as_tensor(test_triplets)
         a, r = ops.as_i32(t[:, 0], dev), ops.as_i32(t[:, 1], dev)
-        idx, score = ops.distmult_topk(embedding, w, a, r, k=topk, shift=flow_log_prob)
+        fp, fi = (None, None) if filter_index is None else filter_index.lists(a, r, "object")
+        idx, score = ops.distmult_topk(embedding, w, a, r, k=topk, shift=flow_log_prob, filt_ptr=fp, filt_idx=fi)
         tails = idx.long()
     if out_path is not None:
         ent = (lambda i: str(entity_names[i])) if entity_names is not None else (lambda i: f"e{i}")
@@ -434,14 +448,15 @@ def generate(embedding, w, test_triplets, eval_bz=200, topk=1, flow_log_prob=Non
             for i in range(len(a_h) if max_lines is None else min(len(a_h), max_lines)):
                 f.write(" - ".join([ent(a_h[i]), rel(r_h[i]), ent(b_h[i])]) + "\n")      # the known triple
                 for c in c_h[i]:
-                    if c != b_h[i]:
+                    if c != b_h[i] and c >= 0:
                         f.write(" = ".join([ent(a_h[i]), rel(r_h[i]), ent(c)]) + "\n")   # a generated one
     return tails, score
 
 
 def build_filter(all_triplets, queries_a, queries_r, num_rels, direction, device):
     """CSR of known-true candidates per query for filtered ranking (extension; the reference is
-    raw-only).  direction "object": candidates c with (a, r, c) known; "subject": (c, r, a)."""
+    raw-only).  direction "object": candidates c with (a, r, c) known; "subject": (c, r, a).
+    Host reference of ``FilterIndex.lists``, which builds the same CSR on the GPU."""
     t = np.asarray(all_triplets)
     key_col, val_col = (0, 2) if direction == "object" else (2, 0)
     keys = t[:, key_col].astype(np.int64) * num_rels + t[:, 1]
@@ -455,6 +470,30 @@ def build_filter(all_triplets, queries_a, queries_r, num_rels, direction, device
     ptr = np.concatenate(([0], np.cumsum([len(x) for x in lists]))).astype(np.int32)
     idx = (np.concatenate(lists) if lists else np.zeros(0)).astype(np.int32)
     return torch.from_numpy(ptr).to(device), torch.from_numpy(idx).to(device)
+
+
+class FilterIndex:
+    """The known triples of a graph (train + valid + test, usually) indexed once per direction on the GPU, for
+    filtered ranks (``calc_mrr(..., filter_index=...)``) and filtered generation (``generate(..., filter_index=...)``).
+    An extension: the reference reports raw ranks only (kgvae/link_predict.py:7).
+
+    ``lists(a, r, direction)`` returns the CSR ``(ptr int32 [M+1], idx int32 [nnz])`` of every entity c with
+    (a_i, r_i, c) known (``direction="object"``) or (c, r_i, a_i) known ("subject"), ascending and duplicate-free:
+    exactly what ``build_filter`` computes on the host, built by the kg_filter_* kernels with one host read-back
+    (the list total).  Ids must lie in [0, num_nodes) / [0, num_rels)."""
+
+    def __init__(self, known_triplets, num_nodes, num_rels, device):
+        device = torch.device(device)
+        if device.type != "cuda":
+            raise RuntimeError("FilterIndex needs a CUDA device (no CPU fallback)")
+        tri = ops.as_i32(known_triplets, device)
+        self.num_nodes, self.num_rels = int(num_nodes), int(num_rels)
+        self.tables = {d: ops.filter_table(tri, self.num_nodes, self.num_rels, d) for d in ops.FILTER_DIRECTIONS}
+
+    def lists(self, a, r, direction):
+        table, n = self.tables[direction]
+        dev = table.device
+        return ops.filter_lists(table, n, self.num_nodes, self.num_rels, ops.as_i32(a, dev), ops.as_i32(r, dev))
 
 
 # --------------------------------------------------------------------------------------------

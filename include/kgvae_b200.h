@@ -445,6 +445,42 @@ int kg_distmult_topk(const float* emb, const float* w, const int32_t* a, const i
                      int n_queries, int n_entities, int h, const float* shift /* device scalar or NULL */,
                      int k, void* workspace, size_t workspace_bytes, int32_t* out_idx, float* out_score,
                      void* stream);
+/* Filtered generation (new; the reference generates from all entities, kgvae/utils.py:245-288): the same, with
+ * every entity of query i's list filt_idx[filt_ptr[i] .. filt_ptr[i+1]) (ascending, duplicate-free - the lists of
+ * kg_filter_gather) excluded; there is no target to exempt.  Fewer than k unlisted entities: trailing -1 entries.
+ * The exclusion happens inside the score-tile epilogue and the finish pass: workspace as kg_distmult_topk. */
+int kg_distmult_topk_filtered(const float* emb, const float* w, const int32_t* a, const int32_t* r,
+                              int n_queries, int n_entities, int h, const float* shift, int k,
+                              const int32_t* filt_ptr, const int32_t* filt_idx, void* workspace,
+                              size_t workspace_bytes, int32_t* out_idx, float* out_score, void* stream);
+
+/* ------------------------------------------------------------------------------------
+ * filter lists for filtered ranks and filtered generation
+ * device counterpart of utils.build_filter, for the filtered forms of perturb_and_get_rank / calc_mrr
+ * (kgvae/utils.py:180-221, 293-314) and generate (:245-288) - an extension: the reference is raw-only
+ * (kgvae/link_predict.py:7)
+ * For a query (a, r): every entity c with (a, r, c) known (KG_FILTER_OBJECT) or (c, r, a) known
+ * (KG_FILTER_SUBJECT), ascending and duplicate-free - the filt_ptr / filt_idx CSR of kg_distmult_rank and
+ * kg_distmult_topk_filtered.  Entity ids in [0, num_nodes), relation ids in [0, num_rels); a query out of range
+ * has an empty list.
+ *   kg_filter_table   known triples [T, 3] (s, r, o) -> table [T] (sorted unique keys (a R + r) N + c) and
+ *                     table_len (device int).  Needs 2 bits(N) + bits(R) <= 64 (wikikg2: 54).
+ *   kg_filter_count   queries (a_i, r_i) -> ptr [M+1]; *total (HOST) = ptr[M], read back once (the call
+ *                     synchronises the stream) so that the caller can allocate idx.  Refuses totals >= 2^31.
+ *   kg_filter_gather  -> idx [total]
+ * ---------------------------------------------------------------------------------- */
+#define KG_FILTER_OBJECT 0
+#define KG_FILTER_SUBJECT 1
+size_t kg_filter_table_workspace_bytes(int n_triples);
+int kg_filter_table(const int32_t* triples, int n_triples, int num_nodes, int num_rels, int direction,
+                    uint64_t* table, int32_t* table_len, void* workspace, size_t workspace_bytes, void* stream);
+size_t kg_filter_count_workspace_bytes(int n_queries);
+int kg_filter_count(const uint64_t* table, const int32_t* table_len, int num_nodes, int num_rels,
+                    const int32_t* a, const int32_t* r, int n_queries, int32_t* ptr, long long* total,
+                    void* workspace, size_t workspace_bytes, void* stream);
+int kg_filter_gather(const uint64_t* table, const int32_t* table_len, int num_nodes, int num_rels,
+                     const int32_t* a, const int32_t* r, int n_queries, const int32_t* ptr, int32_t* idx,
+                     void* stream);
 
 /* Precision of the tensor-core products behind kg_gemm_f32 and kg_distmult_rank (new; the reference runs
  * fp32 library kernels, kgvae/utils.py:200-205, kgvae/flow_network.py:15).  3 (default): the fp32-accurate

@@ -90,6 +90,7 @@ _SIGNATURES = {
     "kg_distmult_topk_workspace_bytes": (_Z, [_I, _I, _I, _I]),
     "kg_distmult_topk": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _I, _P, _Z, _P, _P, _P]),
     "kg_distmult_topk_filtered": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _I, _P, _P, _P, _Z, _P, _P, _P]),
+    "kg_distmult_topk_shard": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _Z, _P, _P, _P]),
     "kg_filter_table_workspace_bytes": (_Z, [_I]),
     "kg_filter_table": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _Z, _P]),
     "kg_filter_count_workspace_bytes": (_Z, [_I]),
@@ -124,7 +125,7 @@ KERNELS_PER_CALL = {
     "kg_sample_relabel": 7, "kg_kl_mog_fwd_rows": 2, "kg_sum_squares_rows": 2,
     "kg_neighbor_sample_plan": 0, "kg_neighbor_sample": 1,
     "kg_kl_mog_fwd": 2, "kg_bce_logits_fwd": 2, "kg_sum_squares": 2, "kg_sum": 2, "kg_distmult_rank": 3, "kg_distmult_topk": 5,
-    "kg_distmult_topk_filtered": 5, "kg_filter_table": 5, "kg_filter_count": 4,
+    "kg_distmult_topk_filtered": 5, "kg_distmult_topk_shard": 5, "kg_filter_table": 5, "kg_filter_count": 4,
 }
 launches = 0          # running count of kernels launched through this binding
 profile = None        # when a dict: name -> [(start_event, end_event), ...] per call

@@ -24,7 +24,7 @@ int kg_fail(int code, const char* fmt, ...) {
 }
 
 extern "C" const char* kg_last_error(void) { return g_err; }
-extern "C" int kg_version(void) { return 101; }
+extern "C" int kg_version(void) { return 102; }
 
 int kg_sm_count() {
   static int cached[64] = {0};            // per device: a process may drive several GPUs

@@ -280,6 +280,10 @@ filter_correction(const float* __restrict__ q32, const float* __restrict__ emb, 
 // tile epilogue, so every tile's list holds its best UNLISTED candidates and the error-band argument above holds
 // for the unlisted entities; the re-scan of a tile skips the listed ones too.  FILT = false is the unfiltered
 // kernel unchanged (the filter fields sit behind the ones it reads).
+// Sharded generation: the candidates are entities [cand_begin, cand_begin + n_cand).  The tiles and their lists
+// use shard-relative ids n; the filter lists hold global ids (compared against cand_begin + n) and the finish pass
+// writes global ids.  The band's |e| maximum is taken over the shard's own candidates, so the argument holds per
+// launch.  Every score is the canonical one, so merging the shards' lists by (score desc, id asc) is exact.
 // ------------------------------------------------------------------------------------------
 struct TopkArgs {
   const float2* colp;
@@ -289,6 +293,7 @@ struct TopkArgs {
   int M, Kp, n_cand, m_tiles, n_tiles, n_terms;
   const int* filt_ptr;   // FILT only
   const int* filt_idx;
+  int cand_begin;
 };
 
 // first position in v[lo, hi) whose value is >= key
@@ -345,21 +350,21 @@ topk_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
 #pragma unroll
       for (int i = 0; i < KK; ++i) { bv[i] = -INFINITY; bi[i] = -1; }
       const float2* cs = colp_s + buf * BN;
-      int fc = 0, fe = 0;            // FILT: cursor into this row's list, at its first id >= n0
+      int fc = 0, fe = 0;            // FILT: cursor into this row's list, at its first id >= cand_begin + n0
       if constexpr (FILT) {
         if (m < p.M) {
           fe = __ldg(p.filt_ptr + m + 1);
-          fc = lower_bound_i32(p.filt_idx, __ldg(p.filt_ptr + m), fe, n0);
+          fc = lower_bound_i32(p.filt_idx, __ldg(p.filt_ptr + m), fe, p.cand_begin + n0);
         }
       }
 #pragma unroll 1
       for (int c = 0; c < BN / 32; ++c) {
         uint32_t v[32];
         tmem_ld_32x32b_x32(taddr + c * 32, v);
-        uint32_t listed = 0;           // FILT: bit j = entity n0 + 32 c + j is listed
+        uint32_t listed = 0;           // FILT: bit j = entity cand_begin + n0 + 32 c + j is listed
         if constexpr (FILT) {
           for (; fc < fe; ++fc) {
-            const int j = __ldg(p.filt_idx + fc) - (n0 + c * 32);
+            const int j = __ldg(p.filt_idx + fc) - (p.cand_begin + n0 + c * 32);
             if (j >= 32) break;
             if (j >= 0) listed |= 1u << j;
           }
@@ -406,13 +411,14 @@ colp_max_kernel(const float2* __restrict__ colp, int n_cand, float* __restrict__
 constexpr int kTopkMax = 10;
 
 // one warp per query; every lane keeps the same sorted list (scores are warp-uniform after the butterfly sum).
+// emb points at the shard's first row (entity cand_begin): the ids n below are shard-relative, the output global.
 // FILT: the tiles' candidate lists hold no listed entity (the epilogue scored them -inf), the re-scan skips them.
 template <bool FILT>
 __global__ void __launch_bounds__(256)
 topk_finish_kernel(const float* __restrict__ q32, const float* __restrict__ emb, const float4* __restrict__ rowp,
                    const float* __restrict__ sqv, const float* __restrict__ cand_v, const int* __restrict__ cand_i,
-                   const float* __restrict__ emax_p, int M, int h, int n_cand, int n_tiles, int KK, int k,
-                   const float* __restrict__ shift_p, int* __restrict__ out_idx, float* __restrict__ out_score,
+                   const float* __restrict__ emax_p, int M, int h, int cand_begin, int n_cand, int n_tiles, int KK,
+                   int k, const float* __restrict__ shift_p, int* __restrict__ out_idx, float* __restrict__ out_score,
                    const int* __restrict__ filt_ptr, const int* __restrict__ filt_idx) {
   const int m = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (m >= M) return;
@@ -453,11 +459,11 @@ topk_finish_kernel(const float* __restrict__ q32, const float* __restrict__ emb,
     const float v_last = __ldg(cv + t * KK + KK - 1);        // the best score NOT kept is <= this one
     if (!(v_last + shift + band >= ts[k - 1])) continue;
     const int n_end = min(n_cand, (t + 1) * BN);
-    int fc = 0, fe = 0, nx = 0x7fffffff;        // FILT: the row's next listed id >= n (warp-uniform)
+    int fc = 0, fe = 0, nx = 0x7fffffff;        // FILT: the row's next listed id >= n, shard-relative (warp-uniform)
     if constexpr (FILT) {
       fe = __ldg(filt_ptr + m + 1);
-      fc = lower_bound_i32(filt_idx, __ldg(filt_ptr + m), fe, t * BN);
-      nx = fc < fe ? __ldg(filt_idx + fc) : 0x7fffffff;
+      fc = lower_bound_i32(filt_idx, __ldg(filt_ptr + m), fe, cand_begin + t * BN);
+      nx = fc < fe ? __ldg(filt_idx + fc) - cand_begin : 0x7fffffff;
     }
     for (int n = t * BN; n < n_end; ++n) {
       if constexpr (FILT) {
@@ -465,7 +471,7 @@ topk_finish_kernel(const float* __restrict__ q32, const float* __restrict__ emb,
         while (nx <= n) {
           listed |= nx == n;
           ++fc;
-          nx = fc < fe ? __ldg(filt_idx + fc) : 0x7fffffff;
+          nx = fc < fe ? __ldg(filt_idx + fc) - cand_begin : 0x7fffffff;
         }
         if (listed) continue;
       }
@@ -474,7 +480,7 @@ topk_finish_kernel(const float* __restrict__ q32, const float* __restrict__ emb,
   }
   if (lane == 0)
     for (int i = 0; i < k; ++i) {
-      out_idx[(size_t)m * k + i] = ti[i] == 0x7fffffff ? -1 : ti[i];
+      out_idx[(size_t)m * k + i] = ti[i] == 0x7fffffff ? -1 : cand_begin + ti[i];
       out_score[(size_t)m * k + i] = ts[i];
     }
 }
@@ -577,18 +583,35 @@ extern "C" size_t kg_distmult_topk_workspace_bytes(int n_queries, int n_entities
   return L.total + kg_align_up(cand * sizeof(float), 1024) + kg_align_up(cand * sizeof(int), 1024) + 2048;
 }
 
-// out_idx [n_queries, k] int32 (entity ids, best first; -1 when fewer than k entities), out_score [n_queries, k]
-// fp32 canonical scores (+ shift): the k highest-scored tails of each query (a_i, r_i) among ALL entities, or among
-// the entities not in the query's filter list (filt_ptr != nullptr).
-static int topk_impl(const float* emb, const float* w, const int32_t* a, const int32_t* r, int n_queries,
-                     int n_entities, int h, const float* shift, int k, const int32_t* filt_ptr,
-                     const int32_t* filt_idx, void* workspace, size_t workspace_bytes, int32_t* out_idx,
-                     float* out_score, void* stream) {
+// fill a [M, k] result with -1 / -inf (an empty shard)
+__global__ void __launch_bounds__(256)
+topk_empty_kernel(long long n, int* __restrict__ out_idx, float* __restrict__ out_score) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i < n) { out_idx[i] = -1; out_score[i] = -INFINITY; }
+}
+
+// out_idx [n_queries, k] int32 (global entity ids, best first; -1 when fewer than k eligible entities),
+// out_score [n_queries, k] fp32 canonical scores (+ shift): the k highest-scored tails of each query (a_i, r_i)
+// among the entities [cand_begin, cand_end), or among those of them not in the query's filter list
+// (filt_ptr != nullptr).
+extern "C" int kg_distmult_topk_shard(const float* emb, const float* w, const int32_t* a, const int32_t* r,
+                                      int n_queries, int n_entities, int h, const float* shift, int k,
+                                      int cand_begin, int cand_end, const int32_t* filt_ptr,
+                                      const int32_t* filt_idx, void* workspace, size_t workspace_bytes,
+                                      int32_t* out_idx, float* out_score, void* stream) {
   KG_REQUIRE(n_queries >= 0 && n_entities > 0 && h > 0, "topk: bad sizes");
   KG_REQUIRE(k >= 1 && k <= kTopkMax, "topk: k must be in 1..10");
+  KG_REQUIRE(0 <= cand_begin && cand_begin <= cand_end && cand_end <= n_entities, "topk: bad candidate shard");
+  KG_REQUIRE((filt_ptr == nullptr) == (filt_idx == nullptr), "topk: filter needs both ptr and idx");
   cudaStream_t st = kg_stream(stream);
-  const int M = n_queries, n_cand = n_entities;
+  const int M = n_queries, n_cand = cand_end - cand_begin;
   if (M == 0) return KG_OK;
+  if (n_cand == 0) {
+    const long long n = (long long)M * k;
+    topk_empty_kernel<<<kg_div_up(n, 256), 256, 0, st>>>(n, out_idx, out_score);
+    KG_LAUNCH_OK();
+    return KG_OK;
+  }
   const Layout L = layout(M, n_cand, h);
   const int KK = topk_kk(k);
   const size_t cand = (size_t)M * L.n_tiles * KK;
@@ -613,7 +636,7 @@ static int topk_impl(const float* emb, const float* w, const int32_t* a, const i
   query_prep<<<kg_div_up((long long)M * 32, 256), 256, 0, st>>>(emb, w, a, r, a, M, h, L.Kp, shift, kMu, q32, acat, rowp, sqv);
   KG_LAUNCH_OK();
   const int n_cols = L.n_tiles * BN;
-  entity_prep<<<kg_div_up((long long)n_cols * 32, 256), 256, 0, st>>>(emb, 0, n_cand, n_cols, h, L.Kp, bcat, colp);
+  entity_prep<<<kg_div_up((long long)n_cols * 32, 256), 256, 0, st>>>(emb, cand_begin, n_cand, n_cols, h, L.Kp, bcat, colp);
   KG_LAUNCH_OK();
   colp_max_kernel<<<1, 256, 0, st>>>(colp, n_cand, emax);
   KG_LAUNCH_OK();
@@ -627,7 +650,7 @@ static int topk_impl(const float* emb, const float* w, const int32_t* a, const i
   args.colp = colp; args.sqv = sqv; args.cand_v = cand_v; args.cand_i = cand_i;
   args.M = M; args.Kp = L.Kp; args.n_cand = n_cand; args.m_tiles = L.m_tiles; args.n_tiles = L.n_tiles;
   args.n_terms = n_terms;
-  args.filt_ptr = filt_ptr; args.filt_idx = filt_idx;
+  args.filt_ptr = filt_ptr; args.filt_idx = filt_idx; args.cand_begin = cand_begin;
   const int total = L.m_tiles * L.n_tiles;
   const int grid = total < kg_sm_count() ? total : kg_sm_count();
 #define KG_TOPK_LAUNCH(KK_, FILT_, SLOT_)                                                                       \
@@ -638,20 +661,23 @@ static int topk_impl(const float* emb, const float* w, const int32_t* a, const i
     topk_tc_kernel<KK_, FILT_><<<grid, THREADS, SMEM_BYTES, st>>>(tm_a, tm_b, args);                            \
   } while (0)
   const int fgrid = kg_div_up((long long)M * 32, 256);
+  const float* emb_c = emb + (size_t)cand_begin * h;
   if (filt_ptr == nullptr) {
     if (KK == 2) KG_TOPK_LAUNCH(2, false, 2);
     else if (KK == 4) KG_TOPK_LAUNCH(4, false, 3);
     else KG_TOPK_LAUNCH(kTopkMax + 1, false, 4);
     KG_LAUNCH_OK();
-    topk_finish_kernel<false><<<fgrid, 256, 0, st>>>(q32, emb, rowp, sqv, cand_v, cand_i, emax, M, h, n_cand,
-                                                     L.n_tiles, KK, k, shift, out_idx, out_score, nullptr, nullptr);
+    topk_finish_kernel<false><<<fgrid, 256, 0, st>>>(q32, emb_c, rowp, sqv, cand_v, cand_i, emax, M, h, cand_begin,
+                                                     n_cand, L.n_tiles, KK, k, shift, out_idx, out_score, nullptr,
+                                                     nullptr);
   } else {
     if (KK == 2) KG_TOPK_LAUNCH(2, true, 6);
     else if (KK == 4) KG_TOPK_LAUNCH(4, true, 7);
     else KG_TOPK_LAUNCH(kTopkMax + 1, true, 8);
     KG_LAUNCH_OK();
-    topk_finish_kernel<true><<<fgrid, 256, 0, st>>>(q32, emb, rowp, sqv, cand_v, cand_i, emax, M, h, n_cand,
-                                                    L.n_tiles, KK, k, shift, out_idx, out_score, filt_ptr, filt_idx);
+    topk_finish_kernel<true><<<fgrid, 256, 0, st>>>(q32, emb_c, rowp, sqv, cand_v, cand_i, emax, M, h, cand_begin,
+                                                    n_cand, L.n_tiles, KK, k, shift, out_idx, out_score, filt_ptr,
+                                                    filt_idx);
   }
 #undef KG_TOPK_LAUNCH
   KG_LAUNCH_OK();
@@ -662,8 +688,8 @@ extern "C" int kg_distmult_topk(const float* emb, const float* w, const int32_t*
                                 int n_queries, int n_entities, int h, const float* shift, int k,
                                 void* workspace, size_t workspace_bytes, int32_t* out_idx, float* out_score,
                                 void* stream) {
-  return topk_impl(emb, w, a, r, n_queries, n_entities, h, shift, k, nullptr, nullptr, workspace, workspace_bytes,
-                   out_idx, out_score, stream);
+  return kg_distmult_topk_shard(emb, w, a, r, n_queries, n_entities, h, shift, k, 0, n_entities, nullptr, nullptr,
+                                workspace, workspace_bytes, out_idx, out_score, stream);
 }
 
 extern "C" int kg_distmult_topk_filtered(const float* emb, const float* w, const int32_t* a, const int32_t* r,
@@ -671,6 +697,6 @@ extern "C" int kg_distmult_topk_filtered(const float* emb, const float* w, const
                                          const int32_t* filt_ptr, const int32_t* filt_idx, void* workspace,
                                          size_t workspace_bytes, int32_t* out_idx, float* out_score, void* stream) {
   KG_REQUIRE(filt_ptr != nullptr && filt_idx != nullptr, "topk filtered: needs both filt_ptr and filt_idx");
-  return topk_impl(emb, w, a, r, n_queries, n_entities, h, shift, k, filt_ptr, filt_idx, workspace, workspace_bytes,
-                   out_idx, out_score, stream);
+  return kg_distmult_topk_shard(emb, w, a, r, n_queries, n_entities, h, shift, k, 0, n_entities, filt_ptr, filt_idx,
+                                workspace, workspace_bytes, out_idx, out_score, stream);
 }

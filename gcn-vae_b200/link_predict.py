@@ -2,13 +2,16 @@
 
 ``LinkPredict`` keeps the constructor, ``forward`` / ``calc_score`` / ``regularization_loss`` /
 ``get_loss`` and the ``w_relation`` parameter.  ``main`` keeps the reference's flags and loop;
-evaluation stays on the GPU (the reference moves the model to the CPU for it).
+evaluation stays on the GPU (the reference moves the model to the CPU for it).  Under ``torchrun`` ``main`` trains one
+replica per GPU and shards validation, testing and generation over the entities (``main``'s docstring).
 """
 import argparse
+import os
 import time
 
 import numpy as np
 import torch
+import torch.distributed as dist
 import torch.nn as nn
 
 from . import datasets, ops, utils
@@ -275,28 +278,88 @@ def _graph_inputs(graph, rel, norm, num_nodes, device):
     return node_id, rel_t, edge_norm
 
 
-def _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t, filter_index=None):
+def _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t, filter_index=None,
+              rank=0, world_size=1):
     """Periodic validation with checkpoints (kgvae/link_predict.py:238-259); returns the best MRR so far.  With
     ``filter_index`` the filtered metrics of the same embedding are printed too; the checkpoint choice stays on the
-    raw MRR, as in the reference."""
+    raw MRR, as in the reference.  With several ranks the ranking is sharded (``_eval_embedding``), every rank returns
+    the same MRR, and only rank 0 prints and writes checkpoints."""
     model.eval()
-    print("start eval")
-    torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file)
-    with torch.no_grad():
-        embed = model(val_graph, val_node_id, val_rel, val_norm)
+    if rank == 0:
+        print("start eval")
+        torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file)
+    embed, shift = _eval_embedding(model, val_graph, val_node_id, val_rel, val_norm, world_size)
+    sharded = world_size > 1
     mrr = utils.calc_mrr(embed, model.w_relation, valid_t, hits=[1, 3, 10],
                          eval_bz=args.eval_batch_size, all_batches=False,
-                         flow_log_prob=model._flow_shift())
+                         flow_log_prob=shift, sharded=sharded)
     if filter_index is not None:
         utils.calc_mrr(embed, model.w_relation, valid_t, hits=[1, 3, 10], eval_bz=args.eval_batch_size,
-                       all_batches=False, flow_log_prob=model._flow_shift(), filter_index=filter_index)
+                       all_batches=False, flow_log_prob=shift, filter_index=filter_index, sharded=sharded)
     model.release_graph()
     if mrr < best_mrr:
-        torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file + "_latest")
+        if rank == 0:
+            torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file + "_latest")
     else:
         best_mrr = mrr
-        torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file)
+        if rank == 0:
+            torch.save({"state_dict": model.state_dict(), "epoch": epoch}, args.model_state_file)
     return best_mrr
+
+
+def _eval_embedding(model, graph, node_id, rel, norm, world_size):
+    """The encoder's embedding of the evaluation graph and the flow shift it goes with.  Every rank runs the encoder,
+    but z is sampled with each rank's own noise, so with several ranks rank 0's embedding and shift are broadcast:
+    the ranks' entity shards are then ranked against one embedding."""
+    with torch.no_grad():
+        embed = model(graph, node_id, rel, norm)
+        shift = model._flow_shift()
+        if world_size > 1:
+            embed = embed.contiguous()
+            dist.broadcast(embed, 0)
+            if shift is not None:
+                shift = shift.detach().reshape(1).clone()
+                dist.broadcast(shift, 0)
+    return embed, shift
+
+
+def _join_process_group(args):
+    """(rank, world_size, device, created) for ``main``.  Inside an initialised default process group (a caller's,
+    e.g. spawned test processes) that group is used and the device is the current CUDA device.  Otherwise, when
+    ``WORLD_SIZE`` > 1 (``torchrun``), an NCCL group is created on ``cuda:LOCAL_RANK`` and ``--gpu`` is ignored;
+    ``created`` tells ``main`` to destroy it.  Without either: one process on ``--gpu``."""
+    if dist.is_available() and dist.is_initialized():
+        return dist.get_rank(), dist.get_world_size(), torch.device("cuda", torch.cuda.current_device()), False
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        device = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
+        torch.cuda.set_device(device)
+        dist.init_process_group("nccl", device_id=device)
+        return dist.get_rank(), dist.get_world_size(), device, True
+    device = torch.device("cuda", max(args.gpu, 0))
+    torch.cuda.set_device(device)
+    return 0, 1, device, False
+
+
+def _broadcast_model(model):
+    """Rank 0's parameters and buffers on every rank (replicas start identical)."""
+    with torch.no_grad():
+        for t in list(model.parameters()) + list(model.buffers()):
+            dist.broadcast(t.data, 0)
+
+
+def rank_seeds(rank, world_size):
+    """Give each rank its own sampling streams, after the model was made identical on every rank.  With P =
+    ``world_size`` > 1 ranks, rank p
+      * torch (CPU and CUDA default generators): ``torch.manual_seed((torch.initial_seed() + p) % 2**64)``;
+      * numpy (the global stream of the host sampler): draws ``base = np.random.randint(0, 2**31 - P)`` - the same
+        draw on every rank when the processes were seeded alike - and reseeds with ``np.random.seed(base + p)``.
+    So identically seeded processes draw different batches, noise and edge-sample banks, and a run is reproducible
+    from its seeds.  P = 1 draws nothing and changes nothing."""
+    if world_size <= 1:
+        return
+    torch.manual_seed((torch.initial_seed() + rank) % (1 << 64))
+    base = int(np.random.randint(0, 2**31 - world_size))
+    np.random.seed(base + rank)
 
 
 def _batch_sampler(args, train_data, num_nodes, num_rels, device):
@@ -338,13 +401,36 @@ def _capturable_sampler(args, train_data, num_rels, device):
 
 
 def main(args):
+    """The training / testing / generation program of kgvae/link_predict.py.
+
+    Under ``torchrun --nproc-per-node N`` (or inside a caller's process group) every process trains one replica on
+    its own GPU: rank 0's parameters are broadcast after construction and loading, each rank draws its own
+    ``--graph-batch-size`` sample (``rank_seeds``; weak scaling), and the gradients are averaged by the all-reduce
+    buckets, eagerly or inside the captured step.  The epoch line (rank 0 only) shows the loss terms averaged over the
+    ranks and rank 0's timings.  Validation, --test-mode and --generate rank or generate against rank 0's embedding
+    with the candidates sharded over the ranks; every rank gets the same result and ``main`` returns the same value
+    everywhere.  Only rank 0 prints and writes checkpoints and result.txt.  A process group created here is destroyed
+    on every exit path."""
     data = datasets.load_data(args.dataset)
-    num_nodes, num_rels = data.num_nodes, data.num_rels
-    train_data, valid_data, test_data = data.train, data.valid, data.test
     if not torch.cuda.is_available():
         raise RuntimeError("kgvae_b200 needs a CUDA device (no CPU fallback)")
-    device = torch.device("cuda", max(args.gpu, 0))
-    torch.cuda.set_device(device)
+    rank, world_size, device, created = _join_process_group(args)
+    steps = []
+    try:
+        return _run(args, data, rank, world_size, device, steps)
+    finally:
+        if world_size > 1:            # a captured step holds NCCL kernels: release it before the group goes
+            for step in steps:
+                step.close()
+        if created:
+            dist.destroy_process_group()
+
+
+def _run(args, data, rank, world_size, device, steps):
+    say = print if rank == 0 else (lambda *a, **k: None)
+    sharded = world_size > 1
+    num_nodes, num_rels = data.num_nodes, data.num_rels
+    train_data, valid_data, test_data = data.train, data.valid, data.test
 
     model_class = KGVAE if args.model_class == "KGVAE" else RGCN
     model = LinkPredict(model_class=model_class, in_dim=num_nodes, h_dim=args.n_hidden,
@@ -368,36 +454,40 @@ def main(args):
     forward_time, backward_time = [], []
 
     if args.test_mode:
-        print("\nstart testing:")
+        say("\nstart testing:")
         checkpoint = torch.load(args.model_state_file, map_location=device)
         test_t = torch.LongTensor(test_data)
         test_graph, test_rel, test_norm = utils.build_test_graph(num_nodes, num_rels, test_t)
         test_node_id, test_rel, test_norm = _graph_inputs(test_graph, test_rel, test_norm, num_nodes, device)
         model.eval()
         model.load_state_dict(checkpoint["state_dict"])
-        print("Using best epoch: {}".format(checkpoint["epoch"]))
-        with torch.no_grad():
-            embed = model(test_graph, test_node_id, test_rel, test_norm)
+        if sharded:
+            _broadcast_model(model)
+        say("Using best epoch: {}".format(checkpoint["epoch"]))
+        embed, shift = _eval_embedding(model, test_graph, test_node_id, test_rel, test_norm, world_size)
         if args.generate:             # kgvae/link_predict.py:181-184: generation instead of ranking
-            tails, scores = utils.generate(embed, model.w_relation, test_t, flow_log_prob=model._flow_shift(),
-                                           out_path="result.txt", filter_index=filter_index)
-            print(f"generated tails for {len(tails)} test queries -> result.txt")
+            tails, scores = utils.generate(embed, model.w_relation, test_t, flow_log_prob=shift,
+                                           out_path="result.txt", filter_index=filter_index, sharded=sharded)
+            say(f"generated tails for {len(tails)} test queries -> result.txt")
             return tails
         mrr = utils.calc_mrr(embed, model.w_relation, test_t, hits=[1, 3, 10],
                              eval_bz=args.eval_batch_size, all_batches=True,
-                             flow_log_prob=model._flow_shift())
+                             flow_log_prob=shift, sharded=sharded)
         if filter_index is not None:
             utils.calc_mrr(embed, model.w_relation, test_t, hits=[1, 3, 10], eval_bz=args.eval_batch_size,
-                           all_batches=True, flow_log_prob=model._flow_shift(), filter_index=filter_index)
+                           all_batches=True, flow_log_prob=shift, filter_index=filter_index, sharded=sharded)
         return mrr
 
-    print("start training...")
+    say("start training...")
     epoch, best_mrr = 0, 0
     if args.load:
-        print(f"Loading checkpoint file {args.model_state_file} for training")
+        say(f"Loading checkpoint file {args.model_state_file} for training")
         checkpoint = torch.load(args.model_state_file, map_location=device)
         model.load_state_dict(checkpoint["state_dict"])
         epoch = checkpoint["epoch"]
+    if sharded:
+        _broadcast_model(model)
+        rank_seeds(rank, world_size)
 
     if args.edge_sampler not in ("uniform", "neighbor"):
         raise ValueError("Sampler type must be either 'uniform' or 'neighbor'.")
@@ -409,6 +499,7 @@ def main(args):
         sampler = _capturable_sampler(args, train_data, num_rels, device)
         captured = CapturedTrainStep(model, optimizer, None, sampler.n, buckets=buckets, grad_norm=args.grad_norm,
                                      warmup=1, sampler=sampler)
+        steps.append(captured)
         epoch += 1                       # the warm-up step that precedes the capture is a training step
 
         def train_step():
@@ -435,20 +526,26 @@ def main(args):
     while True:
         model.train()
         epoch += 1
-        (loss, pred_loss, kl, mmd), t_forward, t_backward = train_step()
+        terms, t_forward, t_backward = train_step()
         forward_time.append(t_forward)
         backward_time.append(t_backward)
-        print("Epoch {:04d} | Loss {:.4f} | Best MRR {:.4f} | pred_loss {:.4f} | kl {:.4f} | mmd {:.4f}".format(
-            epoch, loss.item(), best_mrr, pred_loss.item(), kl.item(), mmd.item()))
+        if sharded:                      # the loss terms averaged over the ranks: one all-reduce
+            terms = torch.stack([t.detach().reshape(()).float() for t in terms])
+            dist.all_reduce(terms)
+            terms = terms / world_size
+        if rank == 0:
+            loss, pred_loss, kl, mmd = (float(t) for t in terms)
+            print("Epoch {:04d} | Loss {:.4f} | Best MRR {:.4f} | pred_loss {:.4f} | kl {:.4f} | mmd {:.4f}".format(
+                epoch, loss, best_mrr, pred_loss, kl, mmd))
         if epoch % args.evaluate_every == 0:
             best_mrr = _validate(model, args, epoch, best_mrr, val_graph, val_node_id, val_rel, val_norm, valid_t,
-                                 filter_index)
+                                 filter_index, rank, world_size)
         if epoch >= args.n_epochs:
             break
 
-    print("training done")
-    print("Mean forward time: {:4f}s".format(np.mean(forward_time)))
-    print("Mean Backward time: {:4f}s".format(np.mean(backward_time)))
+    say("training done")
+    say("Mean forward time: {:4f}s".format(np.mean(forward_time)))
+    say("Mean Backward time: {:4f}s".format(np.mean(backward_time)))
     return best_mrr
 
 
@@ -498,5 +595,6 @@ def build_parser():
 
 if __name__ == "__main__":
     parsed = build_parser().parse_args()
-    print(parsed)
+    if int(os.environ.get("RANK", "0")) == 0:
+        print(parsed)
     main(parsed)

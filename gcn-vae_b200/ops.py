@@ -1001,12 +1001,14 @@ def distmult_rank(emb, w, a, r, b, shift=None, cand_range=None, filt_ptr=None, f
     return ranks[:M]
 
 
-def distmult_topk(emb, w, a, r, k=1, shift=None, filt_ptr=None, filt_idx=None):
+def distmult_topk(emb, w, a, r, k=1, shift=None, filt_ptr=None, filt_idx=None, cand_range=None):
     """The ``k`` highest-scored tails of each query (a_i, r_i) among all entities, best first (ties by ascending
     entity id): utils.generate's ``score.argmax`` (kgvae/utils.py:245-288) generalised to top-k, without the
     score matrix.  ``filt_ptr`` / ``filt_idx``: per-query CSR of entities to leave out (ascending, duplicate-free;
     ``filter_lists``); a query with fewer than k other entities gets trailing -1.
-    Returns (idx int32 [M, k], score fp32 [M, k])."""
+    ``cand_range=(lo, hi)``: only entities [lo, hi) are candidates (one shard of a multi-GPU generation; the ids
+    returned are global and the scores the same bits the unsharded call gives, so ``parallel.merge_topk`` of the
+    shards' lists is exact).  Returns (idx int32 [M, k], score fp32 [M, k]), -1 / -inf past the eligible ones."""
     if (filt_ptr is None) != (filt_idx is None):
         raise ValueError("distmult_topk: a filter needs both filt_ptr and filt_idx")
     emb, w = _c(emb.detach()), _c(w.detach())
@@ -1014,14 +1016,11 @@ def distmult_topk(emb, w, a, r, k=1, shift=None, filt_ptr=None, filt_idx=None):
     dev = emb.device
     idx = torch.empty((max(M, 1), k), dtype=torch.int32, device=dev)
     score = torch.empty((max(M, 1), k), dtype=torch.float32, device=dev)
-    ws = L.workspace(L.lib().kg_distmult_topk_workspace_bytes(M, V, h, k), dev)
+    lo, hi = (0, V) if cand_range is None else (int(cand_range[0]), int(cand_range[1]))
+    ws = L.workspace(L.lib().kg_distmult_topk_workspace_bytes(M, hi - lo, h, k), dev)
     sh = None if shift is None else _c(torch.as_tensor(shift, dtype=torch.float32, device=dev).reshape(1))
-    head = (L.f32(emb), L.f32(w), L.i32(a), L.i32(r), M, V, h, L.f32(sh), int(k))
-    tail = (L.ptr(ws), ws.numel(), L.i32(idx), L.f32(score), L.stream())
-    if filt_ptr is None:
-        L.call("kg_distmult_topk", *head, *tail)
-    else:
-        L.call("kg_distmult_topk_filtered", *head, L.i32(filt_ptr), L.i32(filt_idx), *tail)
+    L.call("kg_distmult_topk_shard", L.f32(emb), L.f32(w), L.i32(a), L.i32(r), M, V, h, L.f32(sh), int(k), lo, hi,
+           L.i32(filt_ptr), L.i32(filt_idx), L.ptr(ws), ws.numel(), L.i32(idx), L.f32(score), L.stream())
     return idx[:M], score[:M]
 
 

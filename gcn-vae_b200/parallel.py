@@ -205,6 +205,38 @@ def sharded_rank_counts(count_fn, num_entities, group=None):
     return counts
 
 
+def merge_topk(idx, score, k, group=None):
+    """Entity-sharded generation: every rank holds the ``[M, k]`` top-k lists (``idx`` global entity ids, -1 for
+    none; ``score``) of the same M queries over its own slice of the candidates.  All-gathers them and keeps, per
+    query, the ``k`` best by (score descending, id ascending); -1 entries are dropped and the result is padded with
+    -1 / -inf.  Exact: the shards are disjoint, every score is the same canonical value whichever rank computes it,
+    and the union of the shards' top-k lists contains the global top-k.  Collective; every rank returns the same
+    ``(idx, score)`` (dtypes and device of the inputs)."""
+    ws = dist.get_world_size(group) if dist.is_initialized() else 1
+    idx, score = idx.contiguous(), score.contiguous()
+    if ws > 1:
+        parts_i = [torch.empty_like(idx) for _ in range(ws)]
+        parts_s = [torch.empty_like(score) for _ in range(ws)]
+        dist.all_gather(parts_i, idx, group=group)
+        dist.all_gather(parts_s, score, group=group)
+        idx, score = torch.cat(parts_i, dim=1), torch.cat(parts_s, dim=1)
+    valid = idx >= 0
+    big = torch.iinfo(idx.dtype).max
+    ids = torch.where(valid, idx, torch.full_like(idx, big))
+    sc = torch.where(valid, score, torch.full_like(score, float("-inf")))
+    # (score desc, id asc): sort by id, then stably by score
+    order = torch.sort(ids, dim=1, stable=True)[1]
+    ids, sc = ids.gather(1, order), sc.gather(1, order)
+    order = torch.sort(sc, dim=1, descending=True, stable=True)[1][:, :k]
+    ids, sc = ids.gather(1, order), sc.gather(1, order)
+    if ids.shape[1] < k:
+        pad = k - ids.shape[1]
+        ids = torch.cat([ids, ids.new_full((ids.shape[0], pad), big)], dim=1)
+        sc = torch.cat([sc, sc.new_full((sc.shape[0], pad), float("-inf"))], dim=1)
+    kept = ids != big
+    return torch.where(kept, ids, torch.full_like(ids, -1)), torch.where(kept, sc, torch.full_like(sc, float("-inf")))
+
+
 def partition_by_destination(src, dst, etype, norm, num_nodes, world_size, uniform=False):
     """Destination-node ownership: returns a list (one entry per rank) of dicts with the owned node
     block ``[lo, hi)``, the rank's edges (every edge with dst in the block, original relative

@@ -9,9 +9,10 @@
 """
 import numpy as np
 import torch
+import torch.distributed as dist
 import torch.nn.functional as F
 
-from . import ops
+from . import ops, parallel
 from .graph import Graph
 
 
@@ -385,18 +386,27 @@ def perturb_and_get_rank(embedding, w, a, r, b, test_size, batch_size=100, all_b
     ranks = ops.distmult_rank(embedding, w, a32, r32, b32, shift=flow_log_prob,
                               cand_range=cand_range, filt_ptr=fp, filt_idx=fi).long()
     if verbose:
-        rr = ranks.float() + 1.0
-        print("ranked {} queries: MR : {:.6f} |  MRR : {:.6f} | Hit1: {:.6f} | Hit5: {:.6f} | Hit10: {:.6f}".format(
-            n, rr.mean().item(), (1.0 / rr).mean().item(), (rr <= 1).float().mean().item(),
-            (rr <= 5).float().mean().item(), (rr <= 10).float().mean().item()))
+        _print_rank_line(ranks)
     return ranks
 
 
+def _print_rank_line(ranks):
+    rr = ranks.float() + 1.0
+    print("ranked {} queries: MR : {:.6f} |  MRR : {:.6f} | Hit1: {:.6f} | Hit5: {:.6f} | Hit10: {:.6f}".format(
+        ranks.numel(), rr.mean().item(), (1.0 / rr).mean().item(), (rr <= 1).float().mean().item(),
+        (rr <= 5).float().mean().item(), (rr <= 10).float().mean().item()))
+
+
 def calc_mrr(embedding, w, test_triplets, hits=[], eval_bz=100, all_batches=True, flow_log_prob=None,
-             verbose=True, return_ranks=False, filter_index=None):
+             verbose=True, return_ranks=False, filter_index=None, sharded=False, group=None):
     """Raw MRR / Hits@k over both perturbation directions (utils.py:293-314).  With ``filter_index`` (a
     ``FilterIndex``) the metrics are filtered instead (an extension; the reference is raw-only): every other
-    entity that forms a known triple with a query is left out of its rank."""
+    entity that forms a known triple with a query is left out of its rank.
+
+    ``sharded=True`` (multi-GPU; collective over ``group``): each rank counts the candidates of its own entity
+    shard (``parallel.entity_shard``) and the counts are summed with ``parallel.sharded_rank_counts``, so every
+    rank returns the same ranks and MRR as one GPU would.  Every rank must pass the same ``embedding``, ``w``,
+    ``flow_log_prob`` and ``test_triplets``; only rank 0 prints."""
     with torch.no_grad():
         s, r, o = test_triplets[:, 0], test_triplets[:, 1], test_triplets[:, 2]
         n = test_triplets.shape[0]
@@ -405,10 +415,23 @@ def calc_mrr(embedding, w, test_triplets, hits=[], eval_bz=100, all_batches=True
             m = n if all_batches else min(int(n), int(eval_bz))       # the queries perturb_and_get_rank ranks
             filt_s = filter_index.lists(o[:m], r[:m], "subject")      # (c, r, o) known
             filt_o = filter_index.lists(s[:m], r[:m], "object")       # (s, r, c) known
-        ranks_s = perturb_and_get_rank(embedding, w, o, r, s, n, eval_bz, all_batches, flow_log_prob, verbose,
-                                       filt=filt_s)
-        ranks_o = perturb_and_get_rank(embedding, w, s, r, o, n, eval_bz, all_batches, flow_log_prob, verbose,
-                                       filt=filt_o)
+        if sharded:
+            verbose = verbose and dist.get_rank(group) == 0
+            V = embedding.shape[0]
+
+            def direction(a, b, filt):
+                count = lambda lo, hi: perturb_and_get_rank(embedding, w, a, r, b, n, eval_bz, all_batches,
+                                                            flow_log_prob, False, filt=filt, cand_range=(lo, hi))
+                ranks = parallel.sharded_rank_counts(count, V, group)
+                if verbose:
+                    _print_rank_line(ranks)
+                return ranks
+            ranks_s, ranks_o = direction(o, s, filt_s), direction(s, o, filt_o)
+        else:
+            ranks_s = perturb_and_get_rank(embedding, w, o, r, s, n, eval_bz, all_batches, flow_log_prob, verbose,
+                                           filt=filt_s)
+            ranks_o = perturb_and_get_rank(embedding, w, s, r, o, n, eval_bz, all_batches, flow_log_prob, verbose,
+                                           filt=filt_o)
         ranks = torch.cat([ranks_s, ranks_o]) + 1
         mrr = torch.mean(1.0 / ranks.float())
         if verbose:
@@ -420,7 +443,7 @@ def calc_mrr(embedding, w, test_triplets, hits=[], eval_bz=100, all_batches=True
 
 
 def generate(embedding, w, test_triplets, eval_bz=200, topk=1, flow_log_prob=None, entity_names=None,
-             relation_names=None, out_path=None, max_lines=None, filter_index=None):
+             relation_names=None, out_path=None, max_lines=None, filter_index=None, sharded=False, group=None):
     """Tail generation (kgvae/utils.py:245-288): for every test triple (a, r, b) the highest-scored tail(s) among
     all entities.  The reference scores 200 queries at a time through the D x E x V tensor, takes
     ``score.argmax`` and prints the triples around one hard-coded entity using name files from the author's home
@@ -431,6 +454,11 @@ def generate(embedding, w, test_triplets, eval_bz=200, topk=1, flow_log_prob=Non
     ``filter_index`` (a ``FilterIndex``; an extension): only tails c for which (a, r, c) is not a known triple are
     returned - generation proposes new facts.  A query with fewer than ``topk`` such tails gets trailing -1.
 
+    ``sharded=True`` (multi-GPU; collective over ``group``): each rank generates from its own entity shard
+    (``parallel.entity_shard``) and the shards' lists are merged with ``parallel.merge_topk``, which is exact, so
+    every rank returns what one GPU would.  Every rank must pass the same ``embedding``, ``w``, ``flow_log_prob``
+    and ``test_triplets``; only rank 0 writes ``out_path``.
+
     Returns (tails int64 [T, topk], scores fp32 [T, topk]) on the embedding's device; ``tails[:, 0]`` is the
     reference's ``highest_scored``."""
     with torch.no_grad():
@@ -438,7 +466,17 @@ def generate(embedding, w, test_triplets, eval_bz=200, topk=1, flow_log_prob=Non
         t = torch.as_tensor(test_triplets)
         a, r = ops.as_i32(t[:, 0], dev), ops.as_i32(t[:, 1], dev)
         fp, fi = (None, None) if filter_index is None else filter_index.lists(a, r, "object")
-        idx, score = ops.distmult_topk(embedding, w, a, r, k=topk, shift=flow_log_prob, filt_ptr=fp, filt_idx=fi)
+        if sharded:
+            rank = dist.get_rank(group)
+            lo, hi = parallel.entity_shard(embedding.shape[0], rank, dist.get_world_size(group))
+            idx, score = ops.distmult_topk(embedding, w, a, r, k=topk, shift=flow_log_prob, filt_ptr=fp,
+                                           filt_idx=fi, cand_range=(lo, hi))
+            idx, score = parallel.merge_topk(idx, score, topk, group)
+            if rank != 0:
+                out_path = None
+        else:
+            idx, score = ops.distmult_topk(embedding, w, a, r, k=topk, shift=flow_log_prob, filt_ptr=fp,
+                                           filt_idx=fi)
         tails = idx.long()
     if out_path is not None:
         ent = (lambda i: str(entity_names[i])) if entity_names is not None else (lambda i: f"e{i}")

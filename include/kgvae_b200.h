@@ -453,6 +453,18 @@ int kg_distmult_topk_filtered(const float* emb, const float* w, const int32_t* a
                               int n_queries, int n_entities, int h, const float* shift, int k,
                               const int32_t* filt_ptr, const int32_t* filt_idx, void* workspace,
                               size_t workspace_bytes, int32_t* out_idx, float* out_score, void* stream);
+/* Sharded generation (new; multi-GPU): the k best tails among the entities [cand_begin, cand_end) only
+ * (0 <= cand_begin <= cand_end <= n_entities), optionally filtered as kg_distmult_topk_filtered (filt_ptr and
+ * filt_idx both NULL or both set; the lists hold global ids).  out_idx holds GLOBAL entity ids; the scores are the
+ * same canonical bits kg_distmult_topk returns for those entities, so the per-shard lists merge exactly by (score
+ * desc, id asc).  Fewer than k eligible entities in the shard (an empty shard included): trailing -1 / -inf.
+ * kg_distmult_topk and kg_distmult_topk_filtered are the shard [0, n_entities).
+ * workspace: kg_distmult_topk_workspace_bytes(n_queries, cand_end - cand_begin, h, k) bytes. */
+int kg_distmult_topk_shard(const float* emb, const float* w, const int32_t* a, const int32_t* r,
+                           int n_queries, int n_entities, int h, const float* shift, int k,
+                           int cand_begin, int cand_end, const int32_t* filt_ptr /* NULL = unfiltered */,
+                           const int32_t* filt_idx, void* workspace, size_t workspace_bytes,
+                           int32_t* out_idx, float* out_score, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * filter lists for filtered ranks and filtered generation
